@@ -30,7 +30,10 @@ L2 flush is needed between launches.
 cannot thread its simulation; SURVEY.md 8(d)); each process runs long enough (>= 65 536 sites at 100 samples, the same
 number of cells at other sample counts) that its start-up cost is below 3 % of its run.
 
-Launch: python bench.py [--gpus N --steps K --warmup W]; for N > 1 via torch.distributed.run.
+Launch: python bench.py [--gpus N --steps K --warmup W]; for N > 1 via torch.distributed.run.  K sets the timed steps of
+the kernel-side loop and of each e2e mode.  `--dump-outputs DIR` writes a fixed, seeded sample of the batches the last timed
+step left in HBM as DIR/<name>.npy (dump_outputs()); the inputs depend only on the arguments, so two builds run with the same
+arguments can be compared array for array.
 """
 import argparse
 import json
@@ -353,6 +356,67 @@ def sub_leg(name, local, stream):
     return out
 
 
+DUMP_SEED, DUMP_SITES, DUMP_SAMPLES = 20260003, 128, 256     # the sample --dump-outputs writes: <= 48 MB for any workload
+
+
+def dump_outputs(leg, out_dir):
+    """--dump-outputs: a fixed, seeded sample of what the timed loop computed in its last launches (the N_SLOTS batches still
+    resident in HBM, oldest first), as out_dir/<name>.npy.  Per sampled site: the global site id and the vgl_site_out values a
+    caller receives (`site_*`); per sampled cell (site x sample): FORMAT/DP and the tag vectors, padded with NaN to 15 genotypes /
+    5 alleles (NaN throughout a skipped site).  Integers are stored as float64, GL / GP / QS / I16 as the float32 bits the
+    kernels wrote."""
+    import numpy as np
+    import torch
+    capi, ctx, B, S = leg.capi, leg.ctx, leg.wl.B, leg.wl.S
+    rng = np.random.default_rng(DUMP_SEED)
+    samples = np.sort(rng.choice(S, min(DUMP_SAMPLES, S), replace=False))
+    fields = [f for f in capi.SITE_DTYPE.names if f not in ("_pad", "g_off", "r_off")]
+    planes = (("gl", "<f4", "g", 15), ("gp", "<f4", "g", 15), ("pl", "<i4", "g", 15),
+              ("ad", "<i4", "r", 5), ("adf", "<i4", "r", 5), ("adr", "<i4", "r", 5))
+    out = {}
+
+    def gather(ptr, typestr, idx):
+        """plane[idx] of a device plane (torch indexes libvgl's memory through the CUDA array interface, no copy of the plane)"""
+        class Plane:
+            __cuda_array_interface__ = {"shape": (int(idx.max()) + 1,), "typestr": typestr, "data": (ptr, False), "version": 3}
+        t = torch.as_tensor(Plane(), device="cuda")
+        return t[torch.from_numpy(idx).cuda()].cpu().numpy()
+
+    for i in range(leg.i - N_SLOTS, leg.i):
+        slot, first = i % N_SLOTS, leg.site - (leg.i - i) * B
+        b = ctx.wait(slot)
+        recs = ctx.copy_sites(slot, b)
+        sites = np.sort(rng.choice(B, min(DUMP_SITES, B), replace=False))
+        part = {"site_id": (first + sites).astype(np.float64)}
+        for f in fields:
+            v = recs[f][sites]
+            part["site_" + f] = v.astype(np.float32 if v.dtype.kind == "f" else np.float64)
+        part["dp"] = gather(b.raw.dp, "<i4", (sites[:, None] * S + samples[None, :]).reshape(-1)).reshape(len(sites), -1).astype(np.float64)
+        for name, typestr, kind, width in planes:
+            ptr = getattr(b.raw, name)
+            if not ptr:
+                continue
+            idx, pos = [], []
+            for k, site in enumerate(sites):
+                r = recs[site]
+                if r["skip_code"] != 0:
+                    continue
+                n = int(r["n_genotypes"] if kind == "g" else r["n_alleles"])
+                off = int(r["g_off"] if kind == "g" else r["r_off"])
+                idx.append((off + samples[:, None] * n + np.arange(n)[None, :]).reshape(-1))
+                pos.append((k * len(samples) * width + np.arange(len(samples))[:, None] * width + np.arange(n)[None, :]).reshape(-1))
+            dt = np.float32 if typestr == "<f4" else np.float64
+            v = np.full(len(sites) * len(samples) * width, np.nan, dt)
+            if idx:
+                v[np.concatenate(pos)] = gather(ptr, typestr, np.concatenate(idx))
+            part[name] = v.reshape(len(sites), len(samples), width)
+        for k, v in part.items():
+            out.setdefault(k, []).append(v)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), np.concatenate(v))
+
+
 def bind_to_gpu_numa_node(torch, local):
     """Pin this process to the CPU cores NVML lists as close to its GPU.  The pinned host buffers are first touched there, so the
     DMA of the result copies ends on the GPU's own socket instead of crossing the inter-socket link (which all ranks would share).
@@ -410,8 +474,12 @@ def gpu_arm(opt):
     wl = Workload(opt.workload)
     B, S, L, K, W = wl.B, wl.S, wl.L, opt.steps, opt.warmup
     cells_per_step = B * S * L
-    # contiguous site range of this rank (weak scaling: every rank simulates (K + W) * L + spare batches of its own)
-    per_rank_sites = ((K + W) * L + 64) * B
+    Le = max(2, min(L, int(opt.e2e_launches)))       # batches per e2e step
+    E_SLOTS = 3
+    e2e_batches_used = max(E_SLOTS, K * Le)           # every e2e mode simulates the same site range from site_next on
+    # contiguous site range of this rank (weak scaling): the kernel leg's N_SLOTS + (K + W) * L batches, the e2e modes' batches
+    # and spare batches (the input-path leg of a one-GPU run) -- disjoint from the other ranks' ranges
+    per_rank_sites = (N_SLOTS + (K + W) * L + e2e_batches_used + 64) * B
     site0 = rank * per_rank_sites
     stream = torch.cuda.Stream()   # an explicit stream: libvgl treats a NULL stream as "use the slot's own"
 
@@ -434,6 +502,8 @@ def gpu_arm(opt):
     launches = leg.ctx.launch_count() - l0
     clk = clocks.stop() if rank == 0 else None
     roof, dev_ms, alg_bytes, g_share, _ = leg.roofline(last, kern_ms / (K * L))
+    if opt.dump_outputs and rank == 0:
+        dump_outputs(leg, opt.dump_outputs)
     gvcf_leg = leg.gvcf_leg(last) if rank == 0 else None
     site_next = leg.site
     leg.close()
@@ -445,9 +515,6 @@ def gpu_arm(opt):
         if rank == 0:
             print(json.dumps({"profiling_only": True, "value": value, "kernel_ms": dev_ms}))
         return
-    Ke = max(2, min(K, 4))
-    Le = max(2, min(L, int(opt.e2e_launches)))       # batches per e2e step
-    E_SLOTS = 3
     streams = [torch.cuda.Stream() for _ in range(E_SLOTS)]
 
     def out_bytes(b):
@@ -497,14 +564,14 @@ def gpu_arm(opt):
         barrier()
         l0 = ctx.launch_count()
         t0 = time.perf_counter()
-        d2h = e2e_batches(ctx, bufs, Ke * Le, site_next, bcf_in)
+        d2h = e2e_batches(ctx, bufs, K * Le, site_next, bcf_in)
         torch.cuda.synchronize()
         ms = (time.perf_counter() - t0) * 1e3     # host wall clock around the user-facing calls (every wait has returned)
         barrier()
         n_launch = ctx.launch_count() - l0
         ms = max_over_ranks(ms)
         ctx.close()
-        return world * Ke * Le * B * S / (ms * 1e-3), d2h, n_launch
+        return world * K * Le * B * S / (ms * 1e-3), d2h, n_launch
 
     e2e_i32, d2h_i32, _ = e2e_run(capi.HOST_I32)
     e2e_nar, d2h_nar, nl_nar = e2e_run(capi.HOST_NARROW)
@@ -537,7 +604,7 @@ def gpu_arm(opt):
             if name != wl.name:
                 configs[name] = sub_leg(name, local, stream)
     if world == 1 and not opt.no_input_path:
-        input_path = input_path_leg(a, gt, hap, B, S, site_next + 64 * B, local, peak_of=measured_peak)
+        input_path = input_path_leg(a, gt, hap, B, S, site_next + e2e_batches_used * B, local, peak_of=measured_peak)
 
     if rank != 0:
         if dist is not None:
@@ -571,7 +638,7 @@ def gpu_arm(opt):
                    "cpus_bound_near_gpu": numa_cpus},
         "roofline": roof, "cpu_baseline": cpu,
         "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": int(B * S * Le), "d2h_bytes_per_step": d2h_bytes * Le,
-                "steps": Ke, "launches_per_step": Le, "gpu_launches": int(e2e_launches), "timer": "host wall clock, max over ranks",
+                "steps": K, "launches_per_step": Le, "gpu_launches": int(e2e_launches), "timer": "host wall clock, max over ranks",
                 "planes": e2e_planes, "narrow_planes": e2e_narrow,
                 "i32_planes": {"value": e2e_i32, "d2h_bytes_per_step": d2h_i32 * Le,
                                "planes": "VGL_HOST_I32: every plane int32/float32 as add_tags() hands them to htslib"},
@@ -727,7 +794,13 @@ def main():
     ap.add_argument("--skip-e2e", action="store_true", help="profiling only: stop after the kernel-side loop")
     ap.add_argument("--e2e-launches", type=int, default=12, help="batches per end-to-end step (the timed region starts and ends with an empty pipeline)")
     ap.add_argument("--workload", default="cfg5", choices=sorted(WORKLOADS))
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a fixed seeded sample of what the last "
+                                                          "launches computed as DIR/<name>.npy (rank 0; --impl b200 only)")
     opt = ap.parse_args()
+    if opt.steps < 1:
+        ap.error("--steps must be at least 1")
+    if opt.dump_outputs and opt.impl != "b200":
+        ap.error("--dump-outputs writes what the GPU path computed; it does not apply to --impl reference")
     opt.warmup = max(opt.warmup, 3) if opt.impl == "b200" else opt.warmup
     if opt.impl == "reference":
         reference_arm(opt)

@@ -1,5 +1,5 @@
-import sys, numpy as np
-sys.path.insert(0, "/root/repo")
+import os, sys, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench
 from vcfgl_b200 import capi
 wl = bench.Workload(sys.argv[1] if len(sys.argv) > 1 else "cfg2")

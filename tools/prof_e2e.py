@@ -1,7 +1,7 @@
 """tools/prof_e2e.py <workload> [mode] -- wall-clock breakdown of the end-to-end loop (fill / submit / wait per batch)"""
-import sys, time
+import os, sys, time
 import numpy as np
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench
 from vcfgl_b200 import capi
 wl = bench.Workload(sys.argv[1] if len(sys.argv) > 1 else "cfg5")
