@@ -247,7 +247,8 @@ typedef struct vgl_batch_out {
      * block records (END, MIN_DP, the founder's alleles and QS, per-sample minima of PL and DP) -- with the seam to the
      * neighbouring batches already stitched: a block open at the end of a batch is held back and comes out (merged, if the
      * next batch continues it) in front of the next batch's records, or from vgl_gvcf_flush() after the last batch.  Batches
-     * must be waited in submission order; bcf_off is NULL in this mode. */
+     * must be waited in submission order (vgl_wait returns VGL_ESTATE for a slot while an older one is still in flight);
+     * bcf_off is NULL in this mode. */
     int32_t n_recs;
 } vgl_batch_out;
 

@@ -181,3 +181,38 @@ class Oracle:
         """d: tests.vgl_dump.SiteDump"""
         return self.site(d.gts, d.depths, d.r_base, d.r_strand, d.r_qs, d.r_adjqs, d.r_eprob, d.tails,
                          d.em_sample, d.em_n, d.em_codes)
+
+
+def check_sites_on_draws(a, S, hap, native, rp, gl_rtol=0.0):
+    """The oracle run on a batch's own draws (vgl_native_draws: `rp`) must give the tags the kernels emitted for that batch:
+    native[i] = Batch.site(i) of site i, hap = int8 [n_sites, 2S] true genotypes.  GL bit for bit, or (gl_rtol > 0) within
+    that relative tolerance where the bits differ.  Returns the number of written sites compared."""
+    orc = Oracle(a, S)
+    off = rp["read_offsets"]
+    n_cmp = 0
+    for i, d in enumerate(native):
+        sl = slice(off[i * S], off[(i + 1) * S])
+        o = orc.site(hap[i], rp["depths"][i * S:(i + 1) * S], rp["bases"][sl], rp["strands"][sl],
+                     None if rp["qs"] is None else rp["qs"][sl].astype(np.int32),
+                     None if rp["adj_qs"] is None else rp["adj_qs"][sl].astype(np.int32),
+                     None if rp["error_probs"] is None else rp["error_probs"][sl],
+                     rp["tail_dists"][sl].astype(np.int32) if a.add_i16 else None)
+        assert o["ret"] == d["skip_code"], i
+        if o["ret"] != 0:
+            continue
+        assert o["n_alleles"] == d["n_alleles"] and o["n_genotypes"] == d["n_genotypes"], i
+        for key in ("pl", "fmt_ad", "fmt_adf", "fmt_adr", "info_ad", "info_adf", "info_adr"):
+            if not getattr(a, "add_" + key) or d.get(key) is None:
+                continue
+            assert np.array_equal(o[key], d[key]), (i, key, o[key], d[key])
+        same = o["gl"].view(np.uint32) == np.ascontiguousarray(d["gl"]).view(np.uint32)   # missing (a NaN payload) compares by bits
+        if gl_rtol > 0:
+            with np.errstate(invalid="ignore"):
+                same |= np.abs(o["gl"].astype(np.float64) - d["gl"]) <= gl_rtol * np.abs(d["gl"].astype(np.float64))
+        assert same.all(), i
+        if a.add_qs:
+            assert np.array_equal(o["qs"].view(np.uint32), np.ascontiguousarray(d["qs"]).view(np.uint32)), i
+        if a.add_i16:
+            assert np.array_equal(o["i16"].view(np.uint32), np.ascontiguousarray(d["i16"]).view(np.uint32)), (i, o["i16"], d["i16"])
+        n_cmp += 1
+    return n_cmp

@@ -37,4 +37,9 @@ void shim_bgzf_code(const uint32_t* hist, int fixed, uint32_t* out)
     memcpy(out, &c, sizeof(c));
 }
 int shim_bgzf_code_words() { return (int)(sizeof(vgl::BgzfCode) / 4); }
+// 1 when exactly n_fmt FORMAT blocks of S samples tile the len bytes at p (the check vgl_submit runs on VGL_HOST_BCF input)
+int shim_bcf_fmt_blocks_tile(const uint8_t* p, uint64_t len, uint32_t n_fmt, int64_t n_samples)
+{
+    return vgl::bcf_fmt_blocks_tile(p, len, n_fmt, n_samples) ? 1 : 0;
+}
 }

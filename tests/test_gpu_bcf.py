@@ -325,3 +325,26 @@ def test_cpp_host_stream_writes_a_bgzf_file(tmp_path):
             a_, b_ = (subprocess.check_output([reader, f]).decode().splitlines() for f in (plain, packed))
             assert a_[0].split()[:4] == ["format", "9", "compression", "0"] and b_[0].split()[:4] == ["format", "9", "compression", "2"]   # bcf; none / bgzf
             assert a_[1:] == b_[1:] and a_[-1] == "records %d" % n_sites
+
+
+def test_input_record_with_fewer_format_blocks_than_n_fmt_is_rejected():
+    # two blocks fill fmt_len exactly but the record promises three: vgl_submit refuses it before any copy or launch
+    # (the host check: tests/test_bcf_input_check.py), and the slot takes the corrected record afterwards
+    a = vargs.parse_args("--seed 1 -d 4 -e 0.01 -GL 1 -addPL 1".split())
+    S = 3
+    ctx = capi.Context(capi.params_from_args(a, S, 4, n_slots=1, host_output=capi.HOST_BCF, bcf_dict=dict(DP=1, GL=2, PL=3),
+                                             bcf_blob_bytes_per_site=64))
+    ctx.input_buffer(0)[:1] = 0
+    sin, blob = ctx.bcf_input(0)
+    sin[:1] = 0
+    fb = bo.enc_int1(60) + bo.enc_vint([10, 20, 30], 1) + bo.enc_int1(61) + bo.enc_size(1, bo.BT_FLOAT) + np.ones(S, "<f4").tobytes()
+    blob[:len(fb)] = np.frombuffer(fb, np.uint8)
+    sin[0]["fmt_off"], sin[0]["fmt_len"], sin[0]["n_fmt"] = 0, len(fb), 3
+    launches = ctx.launch_count()
+    with pytest.raises(capi.VglError) as e:
+        ctx.submit(0, 0, 1)
+    assert e.value.code == capi.VGL_EINVAL and ctx.launch_count() == launches
+    sin[0]["n_fmt"] = 2
+    ctx.submit(0, 0, 1)
+    assert ctx.wait(0).status == 0
+    ctx.close()

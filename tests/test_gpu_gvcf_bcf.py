@@ -23,9 +23,15 @@ def all_sites(cid):
     return gc.case_sites(cid) if cid in gu.MAIN_GVCF else gu.vgl_dump.read_dump(gu.os.path.join(gu.GVCF_DIR, cid + ".vgld.gz"))
 
 
-@pytest.mark.parametrize("batch", [0, 1, 7, 13])
+# (batch size, slots): with three slots, up to three batches are in flight before the first wait (the seam is stitched in
+# vgl_wait, in submission order)
+BATCHES = [pytest.param(0, 1, id="0"), pytest.param(1, 1, id="1"), pytest.param(7, 1, id="7"), pytest.param(13, 1, id="13"),
+           pytest.param(7, 3, id="7-slots3"), pytest.param(13, 3, id="13-slots3")]
+
+
+@pytest.mark.parametrize("batch,n_slots", BATCHES)
 @pytest.mark.parametrize("cid", gu.CASES)
-def test_gvcf_record_stream_equals_the_reference_file(cid, batch):
+def test_gvcf_record_stream_equals_the_reference_file(cid, batch, n_slots):
     a, kept, (_, ids, recs) = gu.load(cid)
     if a.do_unobserved not in (1, 2):
         pytest.skip("the reference itself stops at the second member of a block with -doUnobserved 4|5")
@@ -37,7 +43,7 @@ def test_gvcf_record_stream_equals_the_reference_file(cid, batch):
     idx = [i for i, d in enumerate(sites) if d.ret == 0]      # written sites -> capture indices
     d_ids = {k.split("/")[1].lower(): v for k, v in ids.items() if k.split("/")[0] in ("FORMAT", "INFO")}
     bcf_dict = {k: d_ids[k] for k in ("dp", "gl", "pl", "gp", "ad", "adf", "adr", "qs", "i16", "end", "min_dp") if k in d_ids}
-    ctx = capi.Context(capi.params_from_args(a, S, max_batch_sites=batch, n_slots=1, host_output=capi.HOST_BCF, bcf_dict=bcf_dict,
+    ctx = capi.Context(capi.params_from_args(a, S, max_batch_sites=batch, n_slots=n_slots, host_output=capi.HOST_BCF, bcf_dict=bcf_dict,
                                              bcf_blob_bytes_per_site=96))
     ctx.set_gvcf_dps(gu.dps_of(a))
     # pass-through fields of the regular records (block records are cleared records): from the reference's own output
@@ -50,12 +56,23 @@ def test_gvcf_record_stream_equals_the_reference_file(cid, batch):
             pt[idx[o["site"]]] = (r["qual_bits"], n_in, r["id_bytes"], r["filter_bytes"] + b"".join(b for _, b in r["infos"][:n_in]))
     got = bytearray()
     n_out = 0
-    for lo in range(0, n, batch):
+    pending = []
+
+    def take():
+        nonlocal n_out
+        b = ctx.wait(pending.pop(0))
+        assert b.status == 0 and b.bcf_off is None
+        got.extend(bytes(b.bcf) if b.bcf is not None else b"")
+        n_out += b.n_recs
+    for j, lo in enumerate(range(0, n, batch)):
+        slot = j % n_slots
+        if len(pending) == n_slots:
+            take()
         part = sites[lo:lo + batch]
         m = len(part)
         gt, rp = replay_util.batch_from_dump(part, a)
-        ctx.input_buffer(0)[:m] = gt
-        sin, blob = ctx.bcf_input(0)
+        ctx.input_buffer(slot)[:m] = gt
+        sin, blob = ctx.bcf_input(slot)
         sin[:m] = 0
         o_ = 0
         for k, d in enumerate(part):
@@ -71,11 +88,10 @@ def test_gvcf_record_stream_equals_the_reference_file(cid, batch):
                     sin[k]["flt_info_off"], sin[k]["flt_info_len"] = o_, len(fi)
                     blob[o_:o_ + len(fi)] = np.frombuffer(fi, np.uint8)
                     o_ += len(fi)
-        ctx.submit(0, lo, m, replay=rp)
-        b = ctx.wait(0)
-        assert b.status == 0 and b.bcf_off is None
-        got += bytes(b.bcf) if b.bcf is not None else b""
-        n_out += b.n_recs
+        ctx.submit(slot, lo, m, replay=rp)
+        pending.append(slot)
+    while pending:
+        take()
     tail = ctx.gvcf_flush()
     got += tail
     n_out += 1 if tail else 0

@@ -236,20 +236,22 @@ __device__ void bgzf_block_ranges(const BgzfArgs& a, int blk, long long b0, int 
     }
 }
 
-// a warp per block: the block's ranges into its slot of rng_g ({ranges, segments, state, -}, then the ranges)
+// a warp per block: the block's ranges into its slot of rng_g ({ranges, segments, state, -}, then the ranges).  The grid is
+// sized on the host's estimate of the batch's blocks; the loop covers the real count (a short batch that carries most of the
+// pass-through blob makes more blocks than its share of sites predicts).
 __global__ void __launch_bounds__(256) k_bgzf_ranges(const BgzfArgs a)
 {
     const long long total = a.totals[3];
     const long long nblk = total > a.in_cap ? 0 : (total + BGZF_IN - 1) / BGZF_IN;
     const int lane = threadIdx.x & 31;
-    const long long blk = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
-    if (blk >= nblk) return;
-    const long long b0 = blk * BGZF_IN;
-    const int L = (int)min((long long)BGZF_IN, total - b0);
-    uint32_t* const g = a.rng_g + (size_t)blk * BGZF_RNG_WORDS;
-    int n_r = 0, n_s = 0, state = 0;
-    bgzf_block_ranges(a, (int)blk, b0, L, lane, g + 4, BGZF_RNG_LIST, n_r, n_s, state);
-    if (lane == 0) { g[0] = (uint32_t)n_r; g[1] = (uint32_t)n_s; g[2] = (uint32_t)state; g[3] = 0u; }
+    for (long long blk = (long long)blockIdx.x * 8 + (threadIdx.x >> 5); blk < nblk; blk += (long long)gridDim.x * 8) {
+        const long long b0 = blk * BGZF_IN;
+        const int L = (int)min((long long)BGZF_IN, total - b0);
+        uint32_t* const g = a.rng_g + (size_t)blk * BGZF_RNG_WORDS;
+        int n_r = 0, n_s = 0, state = 0;
+        bgzf_block_ranges(a, (int)blk, b0, L, lane, g + 4, BGZF_RNG_LIST, n_r, n_s, state);
+        if (lane == 0) { g[0] = (uint32_t)n_r; g[1] = (uint32_t)n_s; g[2] = (uint32_t)state; g[3] = 0u; }
+    }
 }
 
 #ifdef BGZF_PROF // development: cycles between the kernel's barriers, summed over blocks (make bgzfprof; tools/prof_bgzf.py)

@@ -32,6 +32,7 @@ struct Slot {
     bool submitted = false;
     bool waited = false;
     int32_t n_sites = 0;
+    int64_t seq = 0; // the context's submit count when this slot was last submitted (the order of the batches in flight)
     // host (pinned)
     uint8_t* h_gt = nullptr;
     vgl_site_out* h_sites = nullptr;
@@ -128,6 +129,7 @@ struct vgl_ctx {
     size_t bcf_headroom = 0;               // bytes in front of a slot's pinned record stream (a re-encoded seam block goes there)
     std::vector<uint8_t> flush_rec;
     cudaEvent_t chain_ev = nullptr;        // kernels of the previous submit are done (see vgl_submit)
+    int64_t submit_seq = 0;                // submits so far (Slot::seq)
     uint32_t* d_crc_pow = nullptr;
     uint32_t *d_qcls = nullptr, *d_m2_cmap = nullptr, *d_qm_cdf = nullptr;
     float *d_m2_pure = nullptr, *d_m2_park = nullptr;
@@ -1054,6 +1056,18 @@ extern "C" int vgl_submit(vgl_ctx* ctx, int slot, int64_t first_site_id, int32_t
     Slot& s = ctx->slots[slot];
     if (s.submitted && !s.waited) return fail(ctx, VGL_ESTATE, "slot still in flight: call vgl_wait first");
     const vgl_params& prm = ctx->prm;
+    if (prm.host_output == VGL_HOST_BCF || prm.host_output == VGL_HOST_BGZF) { // the input records, before anything is copied or launched
+        const int64_t S = prm.n_samples;
+        for (int32_t i = 0; i < n_sites; ++i) { // byte ranges must lie inside the blob
+            const vgl_bcf_site_in& b = s.h_bcf_in[i];
+            if ((size_t)b.id_off + b.id_len > ctx->blob_cap || (size_t)b.flt_info_off + b.flt_info_len > ctx->blob_cap ||
+                (size_t)b.fmt_off + b.fmt_len > ctx->blob_cap)
+                return fail(ctx, VGL_EINVAL, "vgl_bcf_site_in: byte range outside the pass-through blob");
+            if (b.n_fmt > 8 || (b.n_fmt == 0) != (b.fmt_len == 0)) return fail(ctx, VGL_EINVAL, "vgl_bcf_site_in: at most 8 input FORMAT blocks, n_fmt and fmt_len both zero or both set");
+            if (b.n_fmt && !bcf_fmt_blocks_tile(s.h_blob + b.fmt_off, b.fmt_len, b.n_fmt, S))
+                return fail(ctx, VGL_EINVAL, "vgl_bcf_site_in: the input FORMAT blocks do not tile fmt_len bytes");
+        }
+    }
     CK(cudaSetDevice(prm.device_id));
     progress(ctx);
     cudaStream_t st = s.stream;
@@ -1104,35 +1118,6 @@ extern "C" int vgl_submit(vgl_ctx* ctx, int slot, int64_t first_site_id, int32_t
     const bool bcf = prm.host_output == VGL_HOST_BCF || bgzf; // the serialiser posts its byte total (and VGL_EOVERFLOW) in the device words
     const bool tile_status = tile_launch && ((ctx->use_tile_m2 && ctx->tile_m2_mode == 2) || narrow || bcf);
     if (bcf) {
-        for (int32_t i = 0; i < n_sites; ++i) { // byte ranges must lie inside the blob
-            const vgl_bcf_site_in& b = s.h_bcf_in[i];
-            if ((size_t)b.id_off + b.id_len > ctx->blob_cap || (size_t)b.flt_info_off + b.flt_info_len > ctx->blob_cap ||
-                (size_t)b.fmt_off + b.fmt_len > ctx->blob_cap)
-                return fail(ctx, VGL_EINVAL, "vgl_bcf_site_in: byte range outside the pass-through blob");
-            if (b.n_fmt > 8 || (b.n_fmt == 0) != (b.fmt_len == 0)) return fail(ctx, VGL_EINVAL, "vgl_bcf_site_in: at most 8 input FORMAT blocks, n_fmt and fmt_len both zero or both set");
-            if (b.n_fmt) { // the blocks must tile the byte range exactly
-                const uint8_t *q = s.h_blob + b.fmt_off, *end = q + b.fmt_len;
-                for (uint32_t k = 0; k < b.n_fmt && q < end; ++k) {
-                    if (end - q < 2) { q = end + 1; break; }
-                    const uint8_t* r = q;
-                    const int tk = *r & 0xF;
-                    r += 1 + (tk == 1 ? 1 : (tk == 2 ? 2 : 4));
-                    if (r >= end) { q = end + 1; break; }
-                    const int d = *r++;
-                    long n = d >> 4;
-                    const int ty = d & 0xF;
-                    if (n == 15) {
-                        if (r >= end) { q = end + 1; break; }
-                        const int tn = *r & 0xF;
-                        n = tn == 1 ? (int8_t)r[1] : (tn == 2 ? (int16_t)(r[1] | (r[2] << 8)) : (int32_t)(r[1] | (r[2] << 8) | (r[3] << 16) | ((uint32_t)r[4] << 24)));
-                        r += 1 + (tn == 1 ? 1 : (tn == 2 ? 2 : 4));
-                    }
-                    const int w = ty == 1 || ty == 7 ? 1 : (ty == 2 ? 2 : (ty == 0 ? 0 : 4));
-                    q = r + (long)S * n * w;
-                }
-                if (q != end) return fail(ctx, VGL_EINVAL, "vgl_bcf_site_in: the input FORMAT blocks do not tile fmt_len bytes");
-            }
-        }
         CK(cudaMemcpyAsync(s.d_bcf_in, s.h_bcf_in, (size_t)n_sites * sizeof(vgl_bcf_site_in), cudaMemcpyHostToDevice, st));
         CK(cudaMemcpyAsync(s.d_blob, s.h_blob, ctx->blob_cap, cudaMemcpyHostToDevice, st));
     }
@@ -1143,7 +1128,9 @@ extern "C" int vgl_submit(vgl_ctx* ctx, int slot, int64_t first_site_id, int32_t
     // Batches run their kernels strictly one after the other, also across slots with streams of their own: left to itself the
     // GPU interleaves the kernels of all batches in flight, they all finish together, and the result copies then run while
     // the SMs idle.  In order, batch k's copies overlap batch k+1's kernels.
-    if (ctx->chain_ev && prm.host_output) CK(cudaStreamWaitEvent(st, ctx->chain_ev, 0));
+    // The chain also holds under VGL_HOST_NONE: the tile kernels' per-CTA scratch rows (d_m2_park, d_cnt_scratch) belong to
+    // the context, so two batches' kernels must never run at the same time.
+    if (ctx->chain_ev) CK(cudaStreamWaitEvent(st, ctx->chain_ev, 0));
     if (fused) {
         // one kernel does everything; its time is reported as VGL_T_EMIT (SIM / SITE / SCAN = 0)
         CK(cudaEventRecord(s.ev[EV_SIM], st));
@@ -1267,7 +1254,7 @@ extern "C" int vgl_submit(vgl_ctx* ctx, int slot, int64_t first_site_id, int32_t
         }
     }
     CK(cudaGetLastError());
-    if (prm.host_output && !bcf) {
+    if (!bcf) {
         CK(cudaEventRecord(s.ev[EV_KDONE], st));
         ctx->chain_ev = s.ev[EV_KDONE];
     }
@@ -1305,6 +1292,7 @@ extern "C" int vgl_submit(vgl_ctx* ctx, int slot, int64_t first_site_id, int32_t
     s.submitted = true;
     s.waited = false;
     s.n_sites = n_sites;
+    s.seq = ++ctx->submit_seq;
     s.had_d2h = false;
     return VGL_OK;
 }
@@ -1313,7 +1301,7 @@ extern "C" int vgl_submit(vgl_ctx* ctx, int slot, int64_t first_site_id, int32_t
 // may run across the seam between two batches (bcf_utils.cpp:711, 719, 790: same contig, pos <= end + 1, same dp range), so the
 // last record of a batch is held back when it is a block, and merged with the next batch's first record when that joins it --
 // the merged record is the one piece encoded on the host (encode_gvcf_block), written into the headroom in front of the stream.
-// Batches must be waited in submission order.
+// Batches must be waited in submission order (vgl_wait rejects any other).
 static void gvcf_seam(vgl_ctx* ctx, Slot& s, vgl_batch_out* out)
 {
     const size_t S = (size_t)ctx->prm.n_samples;
@@ -1390,6 +1378,9 @@ extern "C" int vgl_wait(vgl_ctx* ctx, int slot, vgl_batch_out* out)
     Slot& s = ctx->slots[slot];
     if (!s.submitted) return fail(ctx, VGL_ESTATE, "slot was not submitted");
     const vgl_params& prm = ctx->prm;
+    if (prm.do_gvcf && prm.host_output == VGL_HOST_BCF && !s.waited) // the seam carries a block from one batch into the next
+        for (const Slot& o : ctx->slots)
+            if (o.submitted && !o.waited && o.seq < s.seq) return fail(ctx, VGL_ESTATE, "-doGVCF: wait for the batches in the order they were submitted");
     CK(cudaSetDevice(prm.device_id));
     // waiting polls, so that the other slots' result copies get enqueued the moment their kernels finish (progress())
     auto wait_event = [&](cudaEvent_t ev) -> cudaError_t {

@@ -607,4 +607,37 @@ void bgzf_build_code(const uint32_t* hist, bool fixed, BgzfCode* out)
     out->hdr_bits = bo.n;
 }
 
+namespace {
+// a BCF typed integer (bcf_enc_int1: type byte, then 1 / 2 / 4 little-endian bytes; other type codes take 4 bytes, as the
+// device's parser reads them, bcf.cu read_typed_int); false when it runs past `end`
+bool read_typed_int(const uint8_t*& p, const uint8_t* end, int64_t& v)
+{
+    if (p >= end) return false;
+    const int t = *p & 0xF, w = t == 1 ? 1 : (t == 2 ? 2 : 4);
+    if (end - p < 1 + w) return false;
+    const uint8_t* r = p + 1;
+    v = w == 1 ? (int8_t)r[0] : (w == 2 ? (int16_t)(r[0] | (r[1] << 8)) : (int32_t)(r[0] | (r[1] << 8) | (r[2] << 16) | ((uint32_t)r[3] << 24)));
+    p += 1 + w;
+    return true;
+}
+} // namespace
+
+bool bcf_fmt_blocks_tile(const uint8_t* p, uint64_t len, uint32_t n_fmt, int64_t n_samples)
+{
+    if (n_samples < 1) return false;
+    const uint8_t* const end = p + len;
+    for (uint32_t k = 0; k < n_fmt; ++k) {
+        int64_t key = 0, n = 0;
+        if (!read_typed_int(p, end, key) || p >= end) return false;
+        const int d = *p++, ty = d & 0xF;
+        n = d >> 4;
+        if (n == 15 && !read_typed_int(p, end, n)) return false;
+        if (n < 0) return false;
+        const uint64_t w = ty == 1 || ty == 7 ? 1 : (ty == 2 ? 2 : (ty == 0 ? 0 : 4)), rest = (uint64_t)(end - p);
+        if (w && n && (uint64_t)n > rest / w / (uint64_t)n_samples) return false; // n x w x S > the bytes left (no overflow)
+        p += (uint64_t)n * w * (uint64_t)n_samples;
+    }
+    return p == end;
+}
+
 } // namespace vgl

@@ -100,4 +100,9 @@ enum { BGZF_HIST = 320 }; // symbol counts: [0..285] literal / length symbols, [
 // fixed = deflate's fixed code; else from the counts (every symbol gets a code, whatever its count)
 void bgzf_build_code(const uint32_t* hist, bool fixed, BgzfCode* out);
 
+// ---- input records of VGL_HOST_BCF (vgl_bcf_site_in): true when exactly n_fmt FORMAT blocks (a typed-integer key, a type
+// descriptor with the vector size, n_samples vectors) tile the `len` bytes at p.  Every byte read lies inside them, and the
+// device's parser (bcf.cu in_fmt_block) then walks n_fmt blocks without leaving the range.
+bool bcf_fmt_blocks_tile(const uint8_t* p, uint64_t len, uint32_t n_fmt, int64_t n_samples);
+
 } // namespace vgl
