@@ -42,4 +42,13 @@ int shim_bcf_fmt_blocks_tile(const uint8_t* p, uint64_t len, uint32_t n_fmt, int
 {
     return vgl::bcf_fmt_blocks_tile(p, len, n_fmt, n_samples) ? 1 : 0;
 }
+// the kernel set vgl_create picks for *p (p->depth_means: the --depths-file means); *status receives plan_run's status
+const char* shim_kernel_set(const vgl_params* p, int allow_tile, int* status)
+{
+    vgl::RunPlan plan;
+    vgl::PlanTables tab;
+    const char* why = "";
+    *status = vgl::plan_run(*p, p->depth_means, allow_tile != 0, &plan, &tab, &why);
+    return vgl::kernel_set_name(plan.set);
+}
 }

@@ -26,6 +26,32 @@ struct DevBuf {
     size_t cap = 0;
 };
 
+// The FORMAT planes of a batch.  GL and GP hold floats, the others int32; both are 4 bytes wide.
+enum { P_DP, P_GL, P_GP, P_PL, P_AD, P_ADF, P_ADR, P_COUNT };
+enum PlaneShape { PER_CELL, PER_GENOTYPE, PER_ALLELE };
+enum PlaneNarrow { NARROW_NONE, NARROW_DEPTH, NARROW_PL }; // VGL_HOST_NARROW: not narrowed, to narrow_bits, to 8 bits (0..255)
+struct PlaneDesc { uint32_t tag; PlaneShape shape; PlaneNarrow narrow; };
+const PlaneDesc kPlanes[P_COUNT] = {
+    {0, PER_CELL, NARROW_DEPTH}, // always there: the kernels write the depths whatever the tags
+    {VGL_TAG_GL, PER_GENOTYPE, NARROW_NONE},
+    {VGL_TAG_GP, PER_GENOTYPE, NARROW_NONE},
+    {VGL_TAG_PL, PER_GENOTYPE, NARROW_PL},
+    {VGL_TAG_FMT_AD, PER_ALLELE, NARROW_DEPTH},
+    {VGL_TAG_FMT_ADF, PER_ALLELE, NARROW_DEPTH},
+    {VGL_TAG_FMT_ADR, PER_ALLELE, NARROW_DEPTH},
+};
+// elements of plane i when the batch has `cells` cells and g / r elements in the G- / R-shaped planes
+size_t plane_elems(int i, size_t cells, size_t g, size_t r)
+{
+    return kPlanes[i].shape == PER_CELL ? cells : kPlanes[i].shape == PER_GENOTYPE ? g : r;
+}
+struct PlaneBufs {
+    void* d = nullptr;  // device, zeroed once at creation
+    void* dn = nullptr; // VGL_HOST_NARROW: device, narrowed
+    void* h = nullptr;  // pinned host: VGL_HOST_I32, and the planes VGL_HOST_NARROW does not narrow
+    void* hn = nullptr; // VGL_HOST_NARROW: pinned host, narrowed
+};
+
 struct Slot {
     cudaStream_t own_stream = nullptr, stream = nullptr;
     cudaEvent_t ev[EV_COUNT] = {};
@@ -37,13 +63,8 @@ struct Slot {
     uint8_t* h_gt = nullptr;
     vgl_site_out* h_sites = nullptr;
     int64_t* h_totals = nullptr; // [0..1] plane extents, [2] status, [3] record-stream bytes, [4] BGZF bytes, [5] BGZF blocks
-    int32_t* h_dp = nullptr;
-    float *h_gl = nullptr, *h_gp = nullptr;
-    int32_t *h_pl = nullptr, *h_ad = nullptr, *h_adf = nullptr, *h_adr = nullptr;
-    // VGL_HOST_NARROW: narrowed integer planes, device and pinned host
-    uint8_t *d_pl8 = nullptr, *h_pl8 = nullptr;
-    void *d_dpn = nullptr, *d_adn = nullptr, *d_adfn = nullptr, *d_adrn = nullptr;
-    void *h_dpn = nullptr, *h_adn = nullptr, *h_adfn = nullptr, *h_adrn = nullptr;
+    PlaneBufs plane[P_COUNT];
+    template <typename T = int32_t> T* dev(int i) const { return static_cast<T*>(plane[i].d); }
     // VGL_HOST_BCF: pass-through input (pinned + device), plan arrays, the record stream (device + pinned)
     vgl_bcf_site_in *h_bcf_in = nullptr, *d_bcf_in = nullptr;
     uint8_t *h_blob = nullptr, *d_blob = nullptr, *d_bcf = nullptr, *h_bcf = nullptr;
@@ -59,7 +80,6 @@ struct Slot {
     int32_t* d_blk_first = nullptr;
     // device
     uint8_t* d_gt = nullptr;
-    int32_t* d_dp = nullptr;
     CellRec* d_cell = nullptr;
     CellQ* d_cellq = nullptr;
     CellTail* d_celltail = nullptr;
@@ -67,8 +87,6 @@ struct Slot {
     int64_t* d_totals = nullptr; // [2] totals, then int32 status at [2]
     uint64_t* d_pairmap = nullptr;
     unsigned long long* d_tile_state = nullptr; // fused: [max tiles] look-back words, then the ticket
-    float *d_gl = nullptr, *d_gp = nullptr;
-    int32_t *d_pl = nullptr, *d_ad = nullptr, *d_adf = nullptr, *d_adr = nullptr;
     // vgl_gvcf_merge(): allocated on first use
     vgl_gvcf_site_in* g_sin = nullptr;
     int2* g_key = nullptr;
@@ -99,16 +117,8 @@ struct Slot {
 struct vgl_ctx {
     vgl_params prm;
     std::vector<double> depth_means;
-    int gl_mode = 0;
-    PreCalc pre;
-    double beta_a = 0, beta_b = 0;
-    int sample_strand = 0, need_cellq = 0, need_tail = 0;
-    uint8_t bin_lut[256];
-    int bin_max = -1;
-    // device tables
-    int use_fused = 0, use_tile = 0, n_sms = 148, fast_div = 0;
-    int tile_aux = 0; // the tile kernel's AUX variant (QS / I16 / INFO ADF, ADR)
-    int use_tile_m2 = 0, tile_m2_mode = 0; // tile_m2.cu; mode 0 / 1 / 2 = --error-qs
+    RunPlan plan; // the run constants and the kernel set (plan_run)
+    int n_sms = 148;
     int narrow_bits = 0;                   // VGL_HOST_NARROW: width of the DP / AD planes (8 or 16), 0 = int32 planes
     size_t bcf_cap = 0, blob_cap = 0;      // VGL_HOST_BCF: bytes per slot of the record stream / the pass-through blob
     int64_t bgzf_max_blocks = 0;           // VGL_HOST_BGZF: blocks a full record stream makes
@@ -134,10 +144,7 @@ struct vgl_ctx {
     uint32_t *d_qcls = nullptr, *d_m2_cmap = nullptr, *d_qm_cdf = nullptr;
     float *d_m2_pure = nullptr, *d_m2_park = nullptr;
     void* d_m1_pure = nullptr;
-    int q_dom = 0, q_dom_idx = 0;
-    double q_minor = 0.0;
     double* d_m2_tab = nullptr;
-    int m2_nq = 0;
     unsigned long long *d_pois = nullptr, *d_alias = nullptr;
     uint16_t* d_alias_row = nullptr; // --depths-file: each sample's row in d_alias
     uint32_t *d_errcdf = nullptr, *d_cnt_scratch = nullptr;
@@ -164,6 +171,12 @@ static int fail(vgl_ctx* ctx, int code, const char* msg)
     return code;
 }
 
+// bytes per element of plane i narrowed (VGL_HOST_NARROW)
+static size_t narrow_bytes(const vgl_ctx* ctx, int i) { return kPlanes[i].narrow == NARROW_PL ? 1 : (size_t)ctx->narrow_bits / 8; }
+
+// kernel sets that run one kernel per batch (a tile state: look-back words and the ticket)
+static bool one_kernel(KernelSet k) { return k == KS_FUSED_M1F || k == KS_TILE_M1F || k == KS_TILE_M2; }
+
 extern "C" int vgl_abi_version(void) { return VGL_ABI_VERSION; }
 
 extern "C" const char* vgl_strerror(int s)
@@ -188,9 +201,7 @@ extern "C" int64_t vgl_launch_count(const vgl_ctx* ctx) { return ctx ? ctx->laun
 
 extern "C" const char* vgl_native_kernels(const vgl_ctx* ctx)
 {
-    if (!ctx) return "";
-    if (ctx->prm.depth_mode == VGL_DEPTH_INF) return "k_truth_site+k_scan+k_truth_emit";
-    return ctx->use_tile ? "k_tile_m1f" : ctx->use_tile_m2 ? "k_tile_m2" : ctx->use_fused ? "k_fused_m1f" : "k_sim+k_site+k_scan+k_emit";
+    return ctx ? kernel_set_name(ctx->plan.set) : "";
 }
 
 extern "C" int64_t vgl_algorithmic_bytes(const vgl_batch_out* o, uint32_t tag_mask)
@@ -258,8 +269,9 @@ static int validate(const vgl_params* p, std::string& why)
 }
 
 template <typename T>
-static cudaError_t upload(T** d, const std::vector<T>& h)
+static cudaError_t upload(T** d, const std::vector<T>& h) // an empty table leaves *d null
 {
+    if (h.empty()) return cudaSuccess;
     cudaError_t e = cudaMalloc((void**)d, h.size() * sizeof(T));
     if (e != cudaSuccess) return e;
     return cudaMemcpy(*d, h.data(), h.size() * sizeof(T), cudaMemcpyHostToDevice);
@@ -278,17 +290,15 @@ extern "C" void vgl_destroy(vgl_ctx* ctx)
         for (auto& e : s.g_ev)
             if (e) cudaEventDestroy(e);
         cudaFree(s.d_disc); cudaFreeHost(s.h_disc);
-        cudaFreeHost(s.h_gt); cudaFreeHost(s.h_sites); cudaFreeHost(s.h_totals); cudaFreeHost(s.h_dp);
-        cudaFreeHost(s.h_gl); cudaFreeHost(s.h_gp); cudaFreeHost(s.h_pl);
-        cudaFreeHost(s.h_ad); cudaFreeHost(s.h_adf); cudaFreeHost(s.h_adr);
-        cudaFreeHost(s.h_pl8); cudaFreeHost(s.h_dpn); cudaFreeHost(s.h_adn); cudaFreeHost(s.h_adfn); cudaFreeHost(s.h_adrn);
+        cudaFreeHost(s.h_gt); cudaFreeHost(s.h_sites); cudaFreeHost(s.h_totals);
+        for (PlaneBufs& b : s.plane) {
+            cudaFree(b.d); cudaFree(b.dn); cudaFreeHost(b.h); cudaFreeHost(b.hn);
+        }
         cudaFreeHost(s.h_bcf_in); cudaFreeHost(s.h_blob); cudaFreeHost(s.h_bcf); cudaFreeHost(s.h_rec_off);
         cudaFree(s.d_bcf_in); cudaFree(s.d_blob); cudaFree(s.d_bcf); cudaFree(s.d_minmax); cudaFree(s.d_rec_len); cudaFree(s.d_rec_off);
         cudaFree(s.d_planes); cudaFree(s.d_stage); cudaFree(s.d_bgzf); cudaFreeHost(s.h_bgzf); cudaFree(s.d_blk_size); cudaFree(s.d_blk_off); cudaFree(s.d_blk_first); cudaFree(s.d_blk_rng);
-        cudaFree(s.d_pl8); cudaFree(s.d_dpn); cudaFree(s.d_adn); cudaFree(s.d_adfn); cudaFree(s.d_adrn);
-        cudaFree(s.d_gt); cudaFree(s.d_dp); cudaFree(s.d_cell); cudaFree(s.d_cellq); cudaFree(s.d_celltail);
+        cudaFree(s.d_gt); cudaFree(s.d_cell); cudaFree(s.d_cellq); cudaFree(s.d_celltail);
         cudaFree(s.d_sites); cudaFree(s.d_totals); cudaFree(s.d_pairmap); cudaFree(s.d_tile_state);
-        cudaFree(s.d_gl); cudaFree(s.d_gp); cudaFree(s.d_pl); cudaFree(s.d_ad); cudaFree(s.d_adf); cudaFree(s.d_adr);
         for (DevBuf* b : {&s.r_depths, &s.r_off, &s.r_bases, &s.r_strands, &s.r_qs, &s.r_adjqs, &s.r_eprob, &s.r_tails, &s.r_deep_cells, &s.r_deep_codes})
             cudaFree(b->p);
         if (s.own_stream) cudaStreamDestroy(s.own_stream);
@@ -306,139 +316,35 @@ static int create_impl(vgl_ctx* ctx)
     if (p.device_id < 0 || p.device_id >= n_dev) return fail(ctx, VGL_EINVAL, "device_id out of range");
     CK(cudaSetDevice(p.device_id));
 
-    // ---- derived run constants (vcfgl.cpp:1661-1766, rng.h:368-371)
-    if (precalc(p.error_rate, p.error_qs, p.gl_model, p.precise_gl, p.adjust_qs, p.adjust_by, p.n_qs_bins, p.qs_bins, &ctx->pre) != 0)
-        return fail(ctx, VGL_ERANGE, "the fixed quality score falls outside every --qs-bins range");
-    if (p.error_qs != 2) ctx->gl_mode = p.gl_model == 1 ? GL_M1_FIXED : GL_M2_FIXED;
-    else ctx->gl_mode = p.gl_model == 1 ? GL_M1_PERREAD : (p.precise_gl ? GL_M2_PRECISE : GL_M2_LUT);
-    if (p.error_qs != 0) {
-        const double m = p.error_rate, one_over = 1.0 / m;
-        ctx->beta_a = (((1.0 - m) / p.beta_variance) - one_over) * pow(m, 2);
-        ctx->beta_b = ctx->beta_a * (one_over - 1);
-        if (!(ctx->beta_a > 0.0) || !(ctx->beta_b > 0.0)) return fail(ctx, VGL_EINVAL, "beta shape parameters must be positive (rng.h:373-388)");
-    }
+    PlanTables tab;
+    const char* why = "";
+    const int rc = plan_run(p, ctx->depth_means.data(), !getenv("VGL_NO_TILE"), &ctx->plan, &tab, &why);
+    if (rc != VGL_OK) return fail(ctx, rc, why);
+    const KernelSet ks = ctx->plan.set;
     const uint32_t t = p.tag_mask;
-    ctx->sample_strand = (t & (VGL_TAG_I16 | VGL_TAG_FMT_ADF | VGL_TAG_FMT_ADR | VGL_TAG_INFO_ADF | VGL_TAG_INFO_ADR)) != 0;
-    ctx->need_cellq = p.error_qs == 2 && (t & (VGL_TAG_QS | VGL_TAG_I16));
-    ctx->need_tail = (t & VGL_TAG_I16) != 0;
-    memset(ctx->bin_lut, 0, sizeof ctx->bin_lut);
-    ctx->bin_max = -1;
-    for (int i = 0; i < p.n_qs_bins; ++i) // first matching range wins (vcfgl.cpp:57-64)
-        for (int q = p.qs_bins[i][0]; q <= p.qs_bins[i][1]; ++q)
-            if (q > ctx->bin_max) { ctx->bin_lut[q] = p.qs_bins[i][2]; ctx->bin_max = q; }
 
     // ---- tables
-    {
-        std::vector<double> lut(&kLutLog10Gl[0][0], &kLutLog10Gl[0][0] + 3 * 257);
-        CK(upload(&ctx->d_lut, lut));
+    CK(upload(&ctx->d_lut, std::vector<double>(&kLutLog10Gl[0][0], &kLutLog10Gl[0][0] + 3 * 257)));
+    CK(upload(&ctx->d_m1_het, tab.m1_het));
+    CK(upload(&ctx->d_m1_bsum, tab.m1_bsum));
+    CK(upload(&ctx->d_fk, tab.fk));
+    CK(upload(&ctx->d_beta, tab.beta));
+    CK(upload(&ctx->d_depth_means, ctx->depth_means));
+    CK(upload(&ctx->d_pois, tab.pois_cdf));
+    ctx->pois_n = (int)tab.pois_cdf.size();
+    CK(cudaDeviceGetAttribute(&ctx->n_sms, cudaDevAttrMultiProcessorCount, p.device_id));
+    if (ks == KS_TILE_M2) {
+        CK(upload(&ctx->d_qcls, tab.qcls));
+        if (p.error_qs == 2) CK(upload(&ctx->d_qm_cdf, binomial_cdf4_u32(ctx->plan.q_minor)));
+        CK(upload(&ctx->d_m2_tab, tab.m2_tab));
+        CK(upload(&ctx->d_m2_cmap, m2_class_map()));
+        CK(upload(&ctx->d_m2_pure, tab.m2_pure));
     }
-    if (p.gl_model == 1) {
-        ErrmodTables em;
-        em.build(1.0 - p.gl1_theta); // io.cpp:1276
-        const std::vector<double> het = em.het_term();
-        CK(upload(&ctx->d_m1_het, het));
-        if (ctx->gl_mode == GL_M1_FIXED) {
-            const int q = (p.adjust_qs & 1) ? ctx->pre.adj_qs : ctx->pre.qs; // gl_methods.cpp:318
-            const std::vector<double> bsum = em.fixed_q_bsum(q);
-            ctx->fast_div = ErrmodTables::scores_safe_for_fast_div(bsum, het) ? 1 : 0;
-            CK(upload(&ctx->d_m1_bsum, bsum));
-        } else {
-            CK(upload(&ctx->d_fk, em.fk));
-            CK(upload(&ctx->d_beta, em.beta));
-        }
-    }
-    if (p.depth_mode == VGL_DEPTH_POISSON_PER_SAMPLE) CK(upload(&ctx->d_depth_means, ctx->depth_means));
-    {
-        cudaDeviceProp prop;
-        CK(cudaGetDeviceProperties(&prop, p.device_id));
-        ctx->n_sms = prop.multiProcessorCount;
-    }
-    // the fused single-kernel path: native RNG, GL model 1 with a run-constant qs, count-level sampler
-    const size_t g_cap_elems = (size_t)p.max_batch_sites * (((size_t)p.n_samples * 15 + 3) & ~(size_t)3);
-    ctx->use_fused = ctx->gl_mode == GL_M1_FIXED && p.sampler != VGL_SAMPLER_PER_READ &&
-                     !(t & (VGL_TAG_QS | VGL_TAG_I16)) && g_cap_elems < (1ull << 31);
-    if (p.sampler == VGL_SAMPLER_COUNTS && !ctx->use_fused) return fail(ctx, VGL_EINVAL, "count-level sampler unavailable for this configuration (plane too large)");
-    // model-2 tile kernel (tile_m2.cu): native RNG, GL model 2 with run constants (--error-qs 0/1) or the qs LUT (--error-qs 2,
-    // --precise-gl 0), tags within GL / PL / AD / DP / INFO AD, DP
-    const uint32_t m2_tags = VGL_TAG_GL | VGL_TAG_PL | VGL_TAG_FMT_AD | VGL_TAG_FMT_DP | VGL_TAG_INFO_AD | VGL_TAG_INFO_DP;
-    const bool m2_cand = p.gl_model == 2 && p.sampler == VGL_SAMPLER_AUTO && !(p.error_qs == 2 && p.precise_gl) && !(t & ~m2_tags) &&
-                         g_cap_elems < (1ull << 31) && p.n_samples <= tile_m1f_max_samples() && !getenv("VGL_NO_TILE");
-    std::vector<unsigned long long> alias(256, 0ull);
-    bool alias_ok = p.depth_mode == VGL_DEPTH_FIXED && p.depth_mean < 256.0;
-    if (p.depth_mode == VGL_DEPTH_POISSON) {
-        const std::vector<unsigned long long> cdf = poisson_cdf_u64(p.depth_mean, 1024);
-        ctx->pois_n = (int)cdf.size();
-        CK(upload(&ctx->d_pois, cdf));
-        const std::vector<unsigned long long> al = poisson_alias_u64(cdf); // empty: depth can exceed 255
-        if (!al.empty()) { alias = al; alias_ok = true; }
-    }
-    std::vector<uint16_t> alias_row;
-    if (p.depth_mode == VGL_DEPTH_POISSON_PER_SAMPLE) { // --depths-file: one alias table per distinct mean, a row index per sample
-        std::vector<double> means;
-        std::vector<unsigned long long> all;
-        alias_ok = true;
-        for (int sidx = 0; sidx < p.n_samples && alias_ok; ++sidx) {
-            const double m = ctx->depth_means[(size_t)sidx];
-            size_t row = 0;
-            while (row < means.size() && means[row] != m) ++row;
-            if (row == means.size()) {
-                const std::vector<unsigned long long> al = poisson_alias_u64(poisson_cdf_u64(m, 1024));
-                if (al.empty() || means.size() >= 65535) { alias_ok = false; break; }
-                means.push_back(m);
-                all.insert(all.end(), al.begin(), al.end());
-            }
-            alias_row.push_back((uint16_t)row);
-        }
-        if (alias_ok) alias = all;
-        else alias_row.clear();
-    }
-    // the tile kernel (tile_m1f.cu): the fused path's headline special case; its AUX variant also takes QS / I16 / INFO ADF, ADR / GP /
-    // FORMAT ADF, ADR
-    const bool tile_base = ctx->gl_mode == GL_M1_FIXED && p.sampler != VGL_SAMPLER_PER_READ && g_cap_elems < (1ull << 31) && alias_ok &&
-                           p.error_qs == 0 && ctx->fast_div &&
-                           p.n_samples <= tile_m1f_max_samples() && !getenv("VGL_NO_TILE");
-    ctx->tile_aux = tile_base && (t & tile_m1f_aux_tags()) != 0;
-    ctx->use_tile = tile_base && (ctx->tile_aux || (ctx->use_fused && !ctx->sample_strand));
-    if (ctx->use_tile) ctx->use_fused = 1; // one launch; the tile kernel replaces k_fused_m1f
-    if (m2_cand && alias_ok) {
-        ctx->tile_m2_mode = p.error_qs;
-        ctx->use_tile_m2 = 1;
-        std::vector<double> consts; // (homT, het, homF) per quality score in use
-        if (p.error_qs == 2) {
-            const bool gl_adj = (p.adjust_qs & 1) != 0;
-            std::vector<int> qv;
-            int dom = 0;
-            const std::vector<uint32_t> qc = qs_class_table(ctx->beta_a, ctx->beta_b, gl_adj ? p.adjust_by : 0.0, p.n_qs_bins > 0, ctx->bin_lut, ctx->bin_max, nullptr, &qv, &dom, &ctx->q_minor);
-            if (qc.empty()) ctx->use_tile_m2 = 0; // classes outside the bins / too many: the per-read kernels keep the reference's behaviour
-            else {
-                CK(upload(&ctx->d_qcls, qc));
-                ctx->q_dom = dom;
-                ctx->q_dom_idx = (int)((qc[256 + dom] >> 16) & 0xFFu);
-                CK(upload(&ctx->d_qm_cdf, binomial_cdf4_u32(ctx->q_minor)));
-            }
-            for (int q : qv) { consts.push_back(kLutLog10Gl[0][q]); consts.push_back(kLutLog10Gl[1][q]); consts.push_back(kLutLog10Gl[2][q]); }
-        } else {
-            consts = {ctx->pre.homT, ctx->pre.het, ctx->pre.homF};
-        }
-        // the table-driven update needs constants that are negative (finite and non-zero, or -inf): see m2_f2d() in tile_m2.cu
-        bool safe = true;
-        for (double c : consts) safe = safe && (c < 0.0);
-        if (ctx->use_tile_m2 && safe) {
-            ctx->m2_nq = (int)consts.size() / 3;
-            CK(upload(&ctx->d_m2_tab, m2_const_table(consts)));
-            CK(upload(&ctx->d_m2_cmap, m2_class_map()));
-            std::vector<float> pure;
-            if (m2_pure_table(consts, &pure)) CK(upload(&ctx->d_m2_pure, pure));
-        } else if (p.error_qs != 2) {
-            ctx->use_tile_m2 = 0; // e.g. --precise-gl 1 with --error-rate 0 (homT = 0): the per-read kernels
-        }
-    }
-    if (p.depth_mode == VGL_DEPTH_INF) ctx->use_fused = ctx->use_tile = ctx->use_tile_m2 = ctx->tile_aux = 0; // truth.cu
     // closed form of cells whose reads all show one base: worth its branch when most 32-cell chunks hold no mis-called read
     // (expected mis-called reads per chunk = 32 x depth x error rate below ~1/2; heterozygous cells are the input's business)
     double exp_depth = p.depth_mode == VGL_DEPTH_POISSON || p.depth_mode == VGL_DEPTH_FIXED ? p.depth_mean : 0.0;
     for (double d : ctx->depth_means) exp_depth = std::max(exp_depth, d);
-    if (ctx->use_tile && 32.0 * exp_depth * p.error_rate < 0.5 && !getenv("VGL_NO_PURE")) {
+    if (ks == KS_TILE_M1F && 32.0 * exp_depth * p.error_rate < 0.5 && !getenv("VGL_NO_PURE")) {
         CK(cudaMalloc(&ctx->d_m1_pure, 256 * sizeof(M1Pure)));
         if (!build_m1f_pure_table(ctx->d_m1_bsum, ctx->d_m1_het, ctx->d_m1_pure, nullptr)) {
             cudaFree(ctx->d_m1_pure);
@@ -446,18 +352,18 @@ static int create_impl(vgl_ctx* ctx)
         }
     }
     // narrow host planes: 8 bits when no cell can hold more than 255 reads (the truncated tail of the Poisson law is below 2^-64)
-    if (p.host_output == VGL_HOST_NARROW) ctx->narrow_bits = alias_ok ? 8 : 16;
-    if (ctx->use_tile || ctx->use_tile_m2) {
-        CK(upload(&ctx->d_alias, alias));
-        if (!alias_row.empty()) CK(upload(&ctx->d_alias_row, alias_row));
+    if (p.host_output == VGL_HOST_NARROW) ctx->narrow_bits = ctx->plan.alias_ok ? 8 : 16;
+    if (ks == KS_TILE_M1F || ks == KS_TILE_M2) {
+        CK(upload(&ctx->d_alias, tab.alias));
+        CK(upload(&ctx->d_alias_row, tab.alias_row));
         CK(upload(&ctx->d_errcdf, binomial_cdf4_u32(p.error_rate)));
-        const size_t words = ctx->use_tile_m2 ? tile_m2_row_words(p.n_samples, ctx->n_sms) : tile_m1f_scratch_words(p.n_samples, ctx->n_sms);
+        const size_t words = ks == KS_TILE_M2 ? tile_m2_row_words(p.n_samples, ctx->n_sms) : tile_m1f_scratch_words(p.n_samples, ctx->n_sms);
         if (words) CK(cudaMalloc((void**)&ctx->d_cnt_scratch, words * 4));
-        if (ctx->use_tile_m2) CK(cudaMalloc((void**)&ctx->d_m2_park, tile_m2_park_floats(p.n_samples, ctx->n_sms) * sizeof(float)));
+        if (ks == KS_TILE_M2) CK(cudaMalloc((void**)&ctx->d_m2_park, tile_m2_park_floats(p.n_samples, ctx->n_sms) * sizeof(float)));
     }
 
     // ---- slots
-    const size_t B = (size_t)p.max_batch_sites, S = (size_t)p.n_samples, cells = B * S;
+    const size_t B = (size_t)p.max_batch_sites, S = (size_t)p.n_samples, cells = B * S, cells4 = (cells + 3) & ~(size_t)3;
     ctx->g_cap = B * ((S * 15 + 3) & ~(size_t)3);
     ctx->r_cap = B * ((S * 5 + 3) & ~(size_t)3);
     ctx->slots.resize(p.n_slots);
@@ -469,48 +375,37 @@ static int create_impl(vgl_ctx* ctx)
         CK(cudaHostAlloc((void**)&s.h_sites, B * sizeof(vgl_site_out), cudaHostAllocDefault));
         CK(cudaHostAlloc((void**)&s.h_totals, 8 * sizeof(int64_t), cudaHostAllocDefault));
         CK(cudaMalloc((void**)&s.d_gt, cells));
-        CK(cudaMalloc((void**)&s.d_dp, cells * sizeof(int32_t)));
         CK(cudaMalloc((void**)&s.d_cell, cells * sizeof(CellRec)));
-        if (ctx->need_cellq) CK(cudaMalloc((void**)&s.d_cellq, cells * sizeof(CellQ)));
-        if (ctx->need_tail) CK(cudaMalloc((void**)&s.d_celltail, cells * sizeof(CellTail)));
+        if (ctx->plan.need_cellq) CK(cudaMalloc((void**)&s.d_cellq, cells * sizeof(CellQ)));
+        if (ctx->plan.need_tail) CK(cudaMalloc((void**)&s.d_celltail, cells * sizeof(CellTail)));
         CK(cudaMalloc((void**)&s.d_sites, B * sizeof(vgl_site_out)));
         CK(cudaMalloc((void**)&s.d_totals, 8 * sizeof(int64_t)));
         CK(cudaMalloc((void**)&s.d_pairmap, B * sizeof(uint64_t)));
-        if (ctx->use_fused || ctx->use_tile_m2) {
+        if (one_kernel(ks)) {
             CK(cudaMalloc((void**)&s.d_tile_state, (B + 2) * sizeof(unsigned long long)));
             CK(cudaMemset(s.d_tile_state, 0, (B + 2) * sizeof(unsigned long long)));
         }
         CK(cudaMemset(s.d_totals, 0, 8 * sizeof(int64_t)));
-        // planes are zeroed once: words the kernels never write (block padding of the general path, tile-end holes) must not
-        // hold another allocation's bits when a whole span is narrowed or copied to the host
-        auto plane = [&](void** d, size_t bytes) -> cudaError_t {
-            cudaError_t e = cudaMalloc(d, bytes);
-            return e != cudaSuccess ? e : cudaMemset(*d, 0, bytes);
-        };
-        if (t & VGL_TAG_GL) CK(plane((void**)&s.d_gl, ctx->g_cap * 4));
-        if (t & VGL_TAG_GP) CK(plane((void**)&s.d_gp, ctx->g_cap * 4));
-        if (t & VGL_TAG_PL) CK(plane((void**)&s.d_pl, ctx->g_cap * 4));
-        if (t & VGL_TAG_FMT_AD) CK(plane((void**)&s.d_ad, ctx->r_cap * 4));
-        if (t & VGL_TAG_FMT_ADF) CK(plane((void**)&s.d_adf, ctx->r_cap * 4));
-        if (t & VGL_TAG_FMT_ADR) CK(plane((void**)&s.d_adr, ctx->r_cap * 4));
-        if (p.host_output == VGL_HOST_NARROW) {
-            const size_t w = (size_t)ctx->narrow_bits / 8, cells4 = (cells + 3) & ~(size_t)3;
-            CK(cudaMalloc(&s.d_dpn, cells4 * w));
-            CK(cudaHostAlloc(&s.h_dpn, cells4 * w, cudaHostAllocDefault));
-            if (t & VGL_TAG_GL) CK(cudaHostAlloc((void**)&s.h_gl, ctx->g_cap * 4, cudaHostAllocDefault));
-            if (t & VGL_TAG_GP) CK(cudaHostAlloc((void**)&s.h_gp, ctx->g_cap * 4, cudaHostAllocDefault));
-            if (t & VGL_TAG_PL) {
-                CK(cudaMalloc((void**)&s.d_pl8, ctx->g_cap));
-                CK(cudaHostAlloc((void**)&s.h_pl8, ctx->g_cap, cudaHostAllocDefault));
+        for (int i = 0; i < P_COUNT; ++i) {
+            if (kPlanes[i].tag && !(t & kPlanes[i].tag)) continue;
+            PlaneBufs& b = s.plane[i];
+            const size_t n = plane_elems(i, cells4, ctx->g_cap, ctx->r_cap);
+            // zeroed once: words the kernels never write (block padding of the general path, tile-end holes) must not hold
+            // another allocation's bits when a whole span is narrowed or copied to the host
+            CK(cudaMalloc(&b.d, n * 4));
+            CK(cudaMemset(b.d, 0, n * 4));
+            if (p.host_output == VGL_HOST_NARROW && kPlanes[i].narrow != NARROW_NONE) {
+                CK(cudaMalloc(&b.dn, n * narrow_bytes(ctx, i)));
+                CK(cudaHostAlloc(&b.hn, n * narrow_bytes(ctx, i), cudaHostAllocDefault));
+            } else if (p.host_output == VGL_HOST_I32 || p.host_output == VGL_HOST_NARROW) {
+                CK(cudaHostAlloc(&b.h, n * 4, cudaHostAllocDefault));
             }
-            if (t & VGL_TAG_FMT_AD) { CK(cudaMalloc(&s.d_adn, ctx->r_cap * w)); CK(cudaHostAlloc(&s.h_adn, ctx->r_cap * w, cudaHostAllocDefault)); }
-            if (t & VGL_TAG_FMT_ADF) { CK(cudaMalloc(&s.d_adfn, ctx->r_cap * w)); CK(cudaHostAlloc(&s.h_adfn, ctx->r_cap * w, cudaHostAllocDefault)); }
-            if (t & VGL_TAG_FMT_ADR) { CK(cudaMalloc(&s.d_adrn, ctx->r_cap * w)); CK(cudaHostAlloc(&s.h_adrn, ctx->r_cap * w, cudaHostAllocDefault)); }
-        } else if (p.host_output == VGL_HOST_BCF || p.host_output == VGL_HOST_BGZF) {
+        }
+        if (p.host_output == VGL_HOST_BCF || p.host_output == VGL_HOST_BGZF) {
             const bool bgzf = p.host_output == VGL_HOST_BGZF;
             // worst case per record: every integer tag at the widest type its values can need (PL <= 255 -> int16; depths
             // bounded by 255 reads under the alias-table law -> int16, else int32) + literals + the pass-through bytes
-            const size_t wc = alias_ok ? 2 : 4, per_site_blob = p.bcf_blob_bytes_per_site ? (size_t)p.bcf_blob_bytes_per_site : 16;
+            const size_t wc = ctx->plan.alias_ok ? 2 : 4, per_site_blob = p.bcf_blob_bytes_per_site ? (size_t)p.bcf_blob_bytes_per_site : 16;
             const size_t per_cell = ((t & VGL_TAG_FMT_DP) ? wc : 0) + ((t & VGL_TAG_GL) ? 60 : 0) + ((t & VGL_TAG_GP) ? 60 : 0) +
                                     ((t & VGL_TAG_PL) ? 30 : 0) + 5 * wc * (!!(t & VGL_TAG_FMT_AD) + !!(t & VGL_TAG_FMT_ADF) + !!(t & VGL_TAG_FMT_ADR));
             ctx->bcf_cap = ((cells * per_cell + B * (512 + per_site_blob)) + 15) & ~(size_t)15;
@@ -551,14 +446,6 @@ static int create_impl(vgl_ctx* ctx)
             CK(cudaMalloc((void**)&s.d_minmax, B * sizeof(BcfSiteMinMax)));
             CK(cudaMalloc((void**)&s.d_rec_len, B * sizeof(uint32_t)));
             CK(cudaMalloc((void**)&s.d_rec_off, (B + 1) * sizeof(long long)));
-        } else if (p.host_output) {
-            CK(cudaHostAlloc((void**)&s.h_dp, cells * sizeof(int32_t), cudaHostAllocDefault));
-            if (t & VGL_TAG_GL) CK(cudaHostAlloc((void**)&s.h_gl, ctx->g_cap * 4, cudaHostAllocDefault));
-            if (t & VGL_TAG_GP) CK(cudaHostAlloc((void**)&s.h_gp, ctx->g_cap * 4, cudaHostAllocDefault));
-            if (t & VGL_TAG_PL) CK(cudaHostAlloc((void**)&s.h_pl, ctx->g_cap * 4, cudaHostAllocDefault));
-            if (t & VGL_TAG_FMT_AD) CK(cudaHostAlloc((void**)&s.h_ad, ctx->r_cap * 4, cudaHostAllocDefault));
-            if (t & VGL_TAG_FMT_ADF) CK(cudaHostAlloc((void**)&s.h_adf, ctx->r_cap * 4, cudaHostAllocDefault));
-            if (t & VGL_TAG_FMT_ADR) CK(cudaHostAlloc((void**)&s.h_adr, ctx->r_cap * 4, cudaHostAllocDefault));
         }
     }
     return VGL_OK;
@@ -630,7 +517,7 @@ extern "C" int vgl_discordance(vgl_ctx* ctx, int slot, vgl_discordance_out* out)
     const vgl_params& prm = ctx->prm;
     Slot& s = ctx->slots[slot];
     if (!s.submitted || !s.waited) return fail(ctx, VGL_ESTATE, "vgl_discordance: call vgl_wait on the slot first");
-    if (!s.d_gl || !(prm.tag_mask & VGL_TAG_FMT_DP) || prm.depth_mode == VGL_DEPTH_INF)
+    if (!s.plane[P_GL].d || !(prm.tag_mask & VGL_TAG_FMT_DP) || prm.depth_mode == VGL_DEPTH_INF)
         return fail(ctx, VGL_EINVAL, "vgl_discordance: needs the GL tag and FORMAT/DP of a simulated batch");
     CK(cudaSetDevice(prm.device_id));
     cudaStream_t st = s.stream;
@@ -641,7 +528,7 @@ extern "C" int vgl_discordance(vgl_ctx* ctx, int slot, vgl_discordance_out* out)
     }
     CK(cudaMemsetAsync(s.d_disc, 0, 4 * sizeof(unsigned long long), st));
     CK(cudaEventRecord(s.g_ev[0], st));
-    launch_discordance(s.d_sites, s.d_gt, s.d_dp, s.d_gl, prm.n_samples, s.n_sites, s.d_disc, st, ctx->n_sms);
+    launch_discordance(s.d_sites, s.d_gt, s.dev(P_DP), s.dev<float>(P_GL), prm.n_samples, s.n_sites, s.d_disc, st, ctx->n_sms);
     ctx->launches += 1;
     CK(cudaGetLastError());
     CK(cudaEventRecord(s.g_ev[1], st));
@@ -670,7 +557,7 @@ static int ensure_gvcf_buffers(vgl_ctx* ctx, Slot& s)
     CK(cudaHostAlloc((void**)&s.hg_counts, 4 * sizeof(int32_t), cudaHostAllocDefault));
     CK(cudaMalloc((void**)&s.g_dp, B * S * sizeof(int32_t)));
     CK(cudaHostAlloc((void**)&s.hg_dp, B * S * sizeof(int32_t), cudaHostAllocDefault));
-    if (s.d_pl) {
+    if (s.plane[P_PL].d) {
         CK(cudaMalloc((void**)&s.g_pl, B * S * 3 * sizeof(int32_t)));
         CK(cudaHostAlloc((void**)&s.hg_pl, B * S * 3 * sizeof(int32_t), cudaHostAllocDefault));
     }
@@ -678,6 +565,19 @@ static int ensure_gvcf_buffers(vgl_ctx* ctx, Slot& s)
 }
 
 // ---- gVCF block merger (gvcf.cu) ----
+static GvcfArgs gvcf_args(const vgl_ctx* ctx, const Slot& s, int32_t n_sites, const int32_t* gvcf_dps, int32_t n_gvcf_dps)
+{
+    GvcfArgs a;
+    memset(&a, 0, sizeof a);
+    a.S = ctx->prm.n_samples, a.n_sites = n_sites;
+    a.dps.n = n_gvcf_dps;
+    for (int i = 0; i < n_gvcf_dps; ++i) a.dps.v[i] = gvcf_dps[i];
+    a.sites = s.d_sites, a.dp = s.dev(P_DP), a.pl = s.dev(P_PL), a.sin = s.g_sin, a.key = s.g_key, a.recs = s.g_recs;
+    a.prev_kept = s.g_prev, a.kept_idx = s.g_kidx, a.counts = s.g_counts, a.out_dp = s.g_dp, a.out_pl = s.g_pl;
+    a.blk_rec = s.g_blast, a.local = s.g_local, a.block_sum = s.g_bsum;
+    return a;
+}
+
 extern "C" int vgl_gvcf_merge(vgl_ctx* ctx, int slot, const vgl_gvcf_site_in* sites, const int32_t* gvcf_dps, int32_t n_gvcf_dps, vgl_gvcf_out* out)
 {
     if (!ctx || !sites || !gvcf_dps || !out || slot < 0 || slot >= (int)ctx->slots.size()) return VGL_EINVAL;
@@ -691,22 +591,14 @@ extern "C" int vgl_gvcf_merge(vgl_ctx* ctx, int slot, const vgl_gvcf_site_in* si
     if (!s.submitted || !s.waited) return fail(ctx, VGL_ESTATE, "vgl_gvcf_merge: call vgl_wait on the slot first");
     if (s.n_sites >= (1 << 21)) return fail(ctx, VGL_EINVAL, "vgl_gvcf_merge: at most 2^21 - 1 sites per batch");
     CK(cudaSetDevice(prm.device_id));
-    const size_t B = (size_t)prm.max_batch_sites, S = (size_t)prm.n_samples;
+    const size_t S = (size_t)prm.n_samples;
     { const int rc = ensure_gvcf_buffers(ctx, s); if (rc != VGL_OK) return rc; }
     if (!s.g_ev[0]) for (auto& e : s.g_ev) CK(cudaEventCreate(&e));
     cudaStream_t st = s.stream;
     const int32_t n = s.n_sites;
     CK(cudaMemcpyAsync(s.g_sin, sites, (size_t)n * sizeof(vgl_gvcf_site_in), cudaMemcpyHostToDevice, st));
-    GvcfArgs a;
-    memset(&a, 0, sizeof a);
-    a.S = (int32_t)S, a.n_sites = n;
-    a.dps.n = n_gvcf_dps;
-    for (int i = 0; i < n_gvcf_dps; ++i) a.dps.v[i] = gvcf_dps[i];
-    a.sites = s.d_sites, a.dp = s.d_dp, a.pl = s.d_pl, a.sin = s.g_sin, a.key = s.g_key, a.recs = s.g_recs;
-    a.prev_kept = s.g_prev, a.kept_idx = s.g_kidx, a.counts = s.g_counts, a.out_dp = s.g_dp, a.out_pl = s.g_pl;
-    a.blk_rec = s.g_blast, a.local = s.g_local, a.block_sum = s.g_bsum;
     CK(cudaEventRecord(s.g_ev[0], st));
-    launch_gvcf(a, st, ctx->n_sms);
+    launch_gvcf(gvcf_args(ctx, s, n, gvcf_dps, n_gvcf_dps), st, ctx->n_sms);
     ctx->launches += 5;
     CK(cudaGetLastError());
     CK(cudaEventRecord(s.g_ev[1], st));
@@ -804,29 +696,29 @@ static void fill_params(const vgl_ctx* ctx, const Slot& s, int64_t first_site_id
     p.depth_means = ctx->d_depth_means;
     p.error_rate = prm.error_rate;
     p.error_qs = prm.error_qs;
-    p.beta_a = ctx->beta_a;
-    p.beta_b = ctx->beta_b;
-    p.gl_mode = ctx->gl_mode;
+    p.beta_a = ctx->plan.beta_a;
+    p.beta_b = ctx->plan.beta_b;
+    p.gl_mode = ctx->plan.gl_mode;
     p.adjust_qs = prm.adjust_qs;
     p.adjust_by = prm.adjust_by;
     p.use_bins = prm.n_qs_bins > 0;
-    p.bin_max = ctx->bin_max;
-    memcpy(p.bin_lut, ctx->bin_lut, 256);
+    p.bin_max = ctx->plan.bin_max;
+    memcpy(p.bin_lut, ctx->plan.bin_lut, 256);
     p.do_unobserved = prm.do_unobserved;
     p.rm_invar_sim = (prm.rm_invar_sites & 4) != 0;
     p.rm_empty = prm.rm_empty_sites != 0;
     p.do_gvcf = prm.do_gvcf != 0;
     p.tag_mask = prm.tag_mask;
     p.i16_mapq = prm.i16_mapq;
-    p.pre_qs = ctx->pre.qs;
-    p.pre_adj_qs = ctx->pre.adj_qs;
-    p.homT = ctx->pre.homT;
-    p.het = ctx->pre.het;
-    p.homF = ctx->pre.homF;
-    p.sample_strand = ctx->sample_strand;
-    p.need_cellq = ctx->need_cellq;
-    p.need_tail = ctx->need_tail;
-    p.fast_div = ctx->fast_div;
+    p.pre_qs = ctx->plan.pre.qs;
+    p.pre_adj_qs = ctx->plan.pre.adj_qs;
+    p.homT = ctx->plan.pre.homT;
+    p.het = ctx->plan.pre.het;
+    p.homF = ctx->plan.pre.homF;
+    p.sample_strand = ctx->plan.sample_strand;
+    p.need_cellq = ctx->plan.need_cellq;
+    p.need_tail = ctx->plan.need_tail;
+    p.fast_div = ctx->plan.fast_div;
     p.zero_holes = prm.host_output == VGL_HOST_I32 || prm.host_output == VGL_HOST_NARROW;
     p.lut_log10 = ctx->d_lut;
     p.m1_bsum = ctx->d_m1_bsum;
@@ -834,7 +726,7 @@ static void fill_params(const vgl_ctx* ctx, const Slot& s, int64_t first_site_id
     p.em_fk = ctx->d_fk;
     p.em_beta = ctx->d_beta;
     p.gt = s.d_gt;
-    p.dp = s.d_dp;
+    p.dp = s.dev(P_DP);
     p.cell = s.d_cell;
     p.cellq = s.d_cellq;
     p.celltail = s.d_celltail;
@@ -851,27 +743,27 @@ static void fill_params(const vgl_ctx* ctx, const Slot& s, int64_t first_site_id
     p.m1_pure = ctx->d_m1_pure;
     p.qcls = ctx->d_qcls;
     p.m2_tab = ctx->d_m2_tab;
-    p.m2_nq = ctx->m2_nq;
+    p.m2_nq = ctx->plan.m2_nq;
     p.m2_cmap = ctx->d_m2_cmap;
     p.qm_cdf = ctx->d_qm_cdf;
-    p.q_minor = ctx->q_minor;
-    p.q_dom = ctx->q_dom;
-    p.q_dom_idx = ctx->q_dom_idx;
+    p.q_minor = ctx->plan.q_minor;
+    p.q_dom = ctx->plan.q_dom;
+    p.q_dom_idx = ctx->plan.q_dom_idx;
     p.m2_pure = ctx->d_m2_pure;
     p.m2_park = ctx->d_m2_park;
     {
         int T = 1024 / (int)S;
         T = T < 1 ? 1 : (T > 128 ? 128 : T);
-        if (ctx->use_tile || ctx->use_tile_m2) T = tile_m1f_sites_per_tile((int)S);
+        const bool tile = ctx->plan.set == KS_TILE_M1F || ctx->plan.set == KS_TILE_M2;
+        if (tile) T = tile_m1f_sites_per_tile((int)S);
         p.sites_per_tile = T;
         p.n_tiles = (n_sites + T - 1) / T;
         p.tile_state = s.d_tile_state;
-        p.ticket = s.d_tile_state ? reinterpret_cast<uint32_t*>(s.d_tile_state + ((ctx->use_tile || ctx->use_tile_m2) ? 0 : p.n_tiles)) : nullptr;
+        p.ticket = s.d_tile_state ? reinterpret_cast<uint32_t*>(s.d_tile_state + (tile ? 0 : p.n_tiles)) : nullptr;
     }
     p.status = reinterpret_cast<int32_t*>(s.d_totals + 2);
-    p.gl = s.d_gl; p.pl = s.d_pl; p.gp = s.d_gp;
-    p.ad = s.d_ad; p.adf = s.d_adf; p.adr = s.d_adr;
-
+    p.gl = s.dev<float>(P_GL); p.pl = s.dev(P_PL); p.gp = s.dev<float>(P_GP);
+    p.ad = s.dev(P_AD); p.adf = s.dev(P_ADF); p.adr = s.dev(P_ADR);
 }
 
 extern "C" int vgl_set_gvcf_dps(vgl_ctx* ctx, const int32_t* gvcf_dps, int32_t n)
@@ -984,19 +876,30 @@ extern "C" int vgl_gvcf_flush(vgl_ctx* ctx, const uint8_t** rec, int64_t* n_byte
     return VGL_OK;
 }
 
+// Copy of n elements of plane i to the host, narrowed when VGL_HOST_NARROW narrows it (nothing when the host has no copy of it)
+static cudaError_t d2h_plane(const vgl_ctx* ctx, const Slot& s, int i, size_t n)
+{
+    const PlaneBufs& b = s.plane[i];
+    if (b.hn) return cudaMemcpyAsync(b.hn, b.dn, n * narrow_bytes(ctx, i), cudaMemcpyDeviceToHost, s.stream);
+    return b.h ? cudaMemcpyAsync(b.h, b.d, n * 4, cudaMemcpyDeviceToHost, s.stream) : cudaSuccess;
+}
+
+// The copies of every plane but DP (it goes with the site records): g / r elements of the G- / R-shaped planes
+static cudaError_t d2h_planes(const vgl_ctx* ctx, const Slot& s, size_t g, size_t r)
+{
+    for (int i = P_DP + 1; i < P_COUNT; ++i) {
+        const cudaError_t e = d2h_plane(ctx, s, i, plane_elems(i, 0, g, r));
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+}
+
 // The result copies of a batch whose extents (plane elements, record bytes, compressed bytes) are only known once its kernels
 // have run: enqueued on the slot's stream as soon as some API call finds the totals on the host.
 static int issue_d2h(vgl_ctx* ctx, Slot& s)
 {
     const vgl_params& prm = ctx->prm;
     cudaStream_t st = s.stream;
-    const int64_t g_elems = s.h_totals[0], r_elems = s.h_totals[1];
-    if (getenv("VGL_TRACE") && s.stream_copied > 0) {
-        float k = 0.f, c = 0.f;
-        cudaEventElapsedTime(&k, s.ev[EV_START], s.ev[EV_D2H0]);
-        cudaEventElapsedTime(&c, s.ev[EV_D2H0], s.ev[EV_D2H1]);
-        fprintf(stderr, "[vgl] slot: start -> kernels done %.2f ms, predicted copy %.2f ms (%.1f MB, %.1f GB/s)\n", k, c, s.stream_copied / 1e6, s.stream_copied / 1e6 / c);
-    }
     CK(cudaEventRecord(s.ev[EV_D2H0], st));
     if (prm.host_output == VGL_HOST_BCF || prm.host_output == VGL_HOST_BGZF) {
         const bool z = prm.host_output == VGL_HOST_BGZF;
@@ -1019,22 +922,8 @@ static int issue_d2h(vgl_ctx* ctx, Slot& s)
             }
         }
         if (nb > 0 && s.n_sites > 0) ctx->stream_bytes_per_site = (double)nb / s.n_sites;
-    } else {
-        if (s.d_gl) CK(cudaMemcpyAsync(s.h_gl, s.d_gl, (size_t)g_elems * 4, cudaMemcpyDeviceToHost, st));
-        if (s.d_gp) CK(cudaMemcpyAsync(s.h_gp, s.d_gp, (size_t)g_elems * 4, cudaMemcpyDeviceToHost, st));
-        if (ctx->narrow_bits) {
-            const size_t w = (size_t)ctx->narrow_bits / 8;
-            if (s.d_pl8) CK(cudaMemcpyAsync(s.h_pl8, s.d_pl8, (size_t)g_elems, cudaMemcpyDeviceToHost, st));
-            if (s.d_adn) CK(cudaMemcpyAsync(s.h_adn, s.d_adn, (size_t)r_elems * w, cudaMemcpyDeviceToHost, st));
-            if (s.d_adfn) CK(cudaMemcpyAsync(s.h_adfn, s.d_adfn, (size_t)r_elems * w, cudaMemcpyDeviceToHost, st));
-            if (s.d_adrn) CK(cudaMemcpyAsync(s.h_adrn, s.d_adrn, (size_t)r_elems * w, cudaMemcpyDeviceToHost, st));
-        } else {
-            if (s.d_pl) CK(cudaMemcpyAsync(s.h_pl, s.d_pl, (size_t)g_elems * 4, cudaMemcpyDeviceToHost, st));
-            if (s.d_ad) CK(cudaMemcpyAsync(s.h_ad, s.d_ad, (size_t)r_elems * 4, cudaMemcpyDeviceToHost, st));
-            if (s.d_adf) CK(cudaMemcpyAsync(s.h_adf, s.d_adf, (size_t)r_elems * 4, cudaMemcpyDeviceToHost, st));
-            if (s.d_adr) CK(cudaMemcpyAsync(s.h_adr, s.d_adr, (size_t)r_elems * 4, cudaMemcpyDeviceToHost, st));
-        }
-    }
+    } else
+        CK(d2h_planes(ctx, s, (size_t)s.h_totals[0], (size_t)s.h_totals[1]));
     CK(cudaEventRecord(s.ev[EV_D2H1], st));
     s.early_d2h = true;
     return VGL_OK;
@@ -1077,15 +966,17 @@ extern "C" int vgl_submit(vgl_ctx* ctx, int slot, int64_t first_site_id, int32_t
     fill_params(ctx, s, first_site_id, n_sites, p);
     CK(cudaEventRecord(s.ev[EV_START], st));
     if (!(flags & VGL_SUBMIT_GT_ON_DEVICE)) CK(cudaMemcpyAsync(s.d_gt, s.h_gt, (size_t)cells, cudaMemcpyHostToDevice, st));
-    const bool tile_launch = (ctx->use_tile || ctx->use_tile_m2) && !rp; // the tile kernel rearms its own ticket and writes the totals itself
+    // a replayed batch runs the general kernels (--depth inf has no draws to replay)
+    const KernelSet ks = rp && ctx->plan.set != KS_TRUTH ? KS_PER_READ : ctx->plan.set;
+    const bool tile_launch = ks == KS_TILE_M1F || ks == KS_TILE_M2; // the tile kernel rearms its own ticket and writes the totals itself
     if (!tile_launch) CK(cudaMemsetAsync(s.d_totals, 0, 8 * sizeof(int64_t), st));
     if (rp) {
         if (!rp->depths || !rp->read_offsets || (rp->n_reads > 0 && !rp->bases)) return fail(ctx, VGL_EINVAL, "replay: depths/read_offsets/bases required");
         if (prm.error_qs == 2 && rp->n_reads > 0 && !rp->qs) return fail(ctx, VGL_EINVAL, "replay: per-read qs required with --error-qs 2");
         if (prm.error_qs == 2 && prm.adjust_qs && rp->n_reads > 0 && !rp->adj_qs) return fail(ctx, VGL_EINVAL, "replay: adjusted qs required with --adjust-qs");
-        if (ctx->gl_mode == GL_M2_PRECISE && rp->n_reads > 0 && !rp->error_probs) return fail(ctx, VGL_EINVAL, "replay: error_probs required with --precise-gl 1");
-        if (ctx->need_tail && rp->n_reads > 0 && !rp->tail_dists) return fail(ctx, VGL_EINVAL, "replay: tail_dists required with -addI16");
-        if (ctx->sample_strand && rp->n_reads > 0 && !rp->strands) return fail(ctx, VGL_EINVAL, "replay: strands required when the strand is sampled");
+        if (ctx->plan.gl_mode == GL_M2_PRECISE && rp->n_reads > 0 && !rp->error_probs) return fail(ctx, VGL_EINVAL, "replay: error_probs required with --precise-gl 1");
+        if (ctx->plan.need_tail && rp->n_reads > 0 && !rp->tail_dists) return fail(ctx, VGL_EINVAL, "replay: tail_dists required with -addI16");
+        if (ctx->plan.sample_strand && rp->n_reads > 0 && !rp->strands) return fail(ctx, VGL_EINVAL, "replay: strands required when the strand is sampled");
         p.replay = 1;
         int rc;
         const size_t nr = (size_t)rp->n_reads;
@@ -1116,13 +1007,13 @@ extern "C" int vgl_submit(vgl_ctx* ctx, int slot, int64_t first_site_id, int32_t
     const bool narrow = prm.host_output == VGL_HOST_NARROW; // the narrowing pass can raise VGL_EOVERFLOW
     const bool bgzf = prm.host_output == VGL_HOST_BGZF;
     const bool bcf = prm.host_output == VGL_HOST_BCF || bgzf; // the serialiser posts its byte total (and VGL_EOVERFLOW) in the device words
-    const bool tile_status = tile_launch && ((ctx->use_tile_m2 && ctx->tile_m2_mode == 2) || narrow || bcf);
+    const bool tile_status = tile_launch && ((ks == KS_TILE_M2 && prm.error_qs == 2) || narrow || bcf);
     if (bcf) {
         CK(cudaMemcpyAsync(s.d_bcf_in, s.h_bcf_in, (size_t)n_sites * sizeof(vgl_bcf_site_in), cudaMemcpyHostToDevice, st));
         CK(cudaMemcpyAsync(s.d_blob, s.h_blob, ctx->blob_cap, cudaMemcpyHostToDevice, st));
     }
     if (tile_status) CK(cudaMemsetAsync(s.d_totals + 2, 0, sizeof(int64_t), st));
-    const bool fused = (ctx->use_fused || ctx->use_tile_m2) && !rp;
+    const bool fused = one_kernel(ks);
     if (fused && !tile_launch) CK(cudaMemsetAsync(s.d_tile_state, 0, ((size_t)p.n_tiles + 1) * sizeof(unsigned long long), st));
     CK(cudaEventRecord(s.ev[EV_H2D], st));
     // Batches run their kernels strictly one after the other, also across slots with streams of their own: left to itself the
@@ -1136,12 +1027,12 @@ extern "C" int vgl_submit(vgl_ctx* ctx, int slot, int64_t first_site_id, int32_t
         CK(cudaEventRecord(s.ev[EV_SIM], st));
         CK(cudaEventRecord(s.ev[EV_SITE], st));
         CK(cudaEventRecord(s.ev[EV_SCAN], st));
-        if (ctx->use_tile) launch_tile_m1f(p, st, ctx->n_sms, ctx->tile_aux != 0);
-        else if (ctx->use_tile_m2) launch_tile_m2(p, st, ctx->n_sms, ctx->tile_m2_mode);
+        if (ks == KS_TILE_M1F) launch_tile_m1f(p, st, ctx->n_sms, ctx->plan.aux);
+        else if (ks == KS_TILE_M2) launch_tile_m2(p, st, ctx->n_sms, prm.error_qs);
         else launch_fused_m1f(p, st, ctx->n_sms);
         CK(cudaEventRecord(s.ev[EV_EMIT], st));
         ctx->launches += 1;
-    } else if (prm.depth_mode == VGL_DEPTH_INF) { // truth.cu: no reads, the tags state the true genotypes
+    } else if (ks == KS_TRUTH) { // truth.cu: no reads, the tags state the true genotypes
         if (rp) return fail(ctx, VGL_EINVAL, "--depth inf has no draws to replay");
         CK(cudaEventRecord(s.ev[EV_SIM], st));
         launch_truth_site(p, st, ctx->n_sms);
@@ -1162,15 +1053,15 @@ extern "C" int vgl_submit(vgl_ctx* ctx, int slot, int64_t first_site_id, int32_t
         CK(cudaEventRecord(s.ev[EV_EMIT], st));
         ctx->launches += 4;
     }
-    if (narrow) { // integer planes -> narrow planes, over the used extents the kernels left in d_totals
-        int32_t* const d_status = reinterpret_cast<int32_t*>(s.d_totals + 2);
-        const int nb = ctx->narrow_bits;
-        launch_narrow(s.d_dp, s.d_dpn, nb, false, nullptr, cells, cells, d_status, st, ctx->n_sms);
-        ctx->launches += 1;
-        if (s.d_pl) { launch_narrow(s.d_pl, s.d_pl8, 8, true, s.d_totals, 0, (int64_t)ctx->g_cap, d_status, st, ctx->n_sms); ctx->launches += 1; }
-        if (s.d_ad) { launch_narrow(s.d_ad, s.d_adn, nb, false, s.d_totals + 1, 0, (int64_t)ctx->r_cap, d_status, st, ctx->n_sms); ctx->launches += 1; }
-        if (s.d_adf) { launch_narrow(s.d_adf, s.d_adfn, nb, false, s.d_totals + 1, 0, (int64_t)ctx->r_cap, d_status, st, ctx->n_sms); ctx->launches += 1; }
-        if (s.d_adr) { launch_narrow(s.d_adr, s.d_adrn, nb, false, s.d_totals + 1, 0, (int64_t)ctx->r_cap, d_status, st, ctx->n_sms); ctx->launches += 1; }
+    if (narrow) { // integer planes -> narrow planes: DP over the batch's cells, the others over the used extents in d_totals
+        for (int i = 0; i < P_COUNT; ++i) {
+            if (!s.plane[i].dn) continue;
+            const bool per_cell = kPlanes[i].shape == PER_CELL;
+            const int64_t* n_dev = per_cell ? nullptr : s.d_totals + (kPlanes[i].shape == PER_ALLELE);
+            launch_narrow(s.dev(i), s.plane[i].dn, (int)narrow_bytes(ctx, i) * 8, kPlanes[i].narrow == NARROW_PL, n_dev, per_cell ? cells : 0,
+                          (int64_t)plane_elems(i, (size_t)cells, ctx->g_cap, ctx->r_cap), reinterpret_cast<int32_t*>(s.d_totals + 2), st, ctx->n_sms);
+            ctx->launches += 1;
+        }
     }
     if (bcf) { // planes -> BCF records (bcf.cu)
         BcfArgs b;
@@ -1178,7 +1069,8 @@ extern "C" int vgl_submit(vgl_ctx* ctx, int slot, int64_t first_site_id, int32_t
         b.S = (int32_t)S; b.n_sites = n_sites; b.tag_mask = prm.tag_mask;
         b.do_unobserved = prm.do_unobserved; b.do_gvcf = prm.do_gvcf; b.dict = prm.bcf_dict;
         b.sites = s.d_sites; b.site_in = s.d_bcf_in; b.blob = s.d_blob;
-        b.dp = s.d_dp; b.gl = s.d_gl; b.gp = s.d_gp; b.pl = s.d_pl; b.ad = s.d_ad; b.adf = s.d_adf; b.adr = s.d_adr;
+        b.dp = s.dev(P_DP); b.gl = s.dev<float>(P_GL); b.gp = s.dev<float>(P_GP); b.pl = s.dev(P_PL);
+        b.ad = s.dev(P_AD); b.adf = s.dev(P_ADF); b.adr = s.dev(P_ADR);
         b.minmax = s.d_minmax; b.rec_len = s.d_rec_len; b.rec_off = s.d_rec_off;
         b.out = s.d_bcf; b.out_cap = (long long)ctx->bcf_cap;
         b.totals = s.d_totals; b.status = reinterpret_cast<int32_t*>(s.d_totals + 2);
@@ -1188,15 +1080,7 @@ extern "C" int vgl_submit(vgl_ctx* ctx, int slot, int64_t first_site_id, int32_t
             if (n_sites >= (1 << 21)) return fail(ctx, VGL_EINVAL, "-doGVCF: at most 2^21 - 1 sites per batch");
             { const int rc2 = ensure_gvcf_buffers(ctx, s); if (rc2 != VGL_OK) return rc2; }
             launch_gvcf_sin_from_bcf(s.d_bcf_in, s.g_sin, n_sites, st);
-            GvcfArgs g;
-            memset(&g, 0, sizeof g);
-            g.S = (int32_t)S, g.n_sites = n_sites;
-            g.dps.n = (int32_t)ctx->gvcf_dps.size();
-            for (int i = 0; i < g.dps.n; ++i) g.dps.v[i] = ctx->gvcf_dps[(size_t)i];
-            g.sites = s.d_sites, g.dp = s.d_dp, g.pl = s.d_pl, g.sin = s.g_sin, g.key = s.g_key, g.recs = s.g_recs;
-            g.prev_kept = s.g_prev, g.kept_idx = s.g_kidx, g.counts = s.g_counts, g.out_dp = s.g_dp, g.out_pl = s.g_pl;
-            g.blk_rec = s.g_blast, g.local = s.g_local, g.block_sum = s.g_bsum;
-            launch_gvcf(g, st, ctx->n_sms);
+            launch_gvcf(gvcf_args(ctx, s, n_sites, ctx->gvcf_dps.data(), (int32_t)ctx->gvcf_dps.size()), st, ctx->n_sms);
             ctx->launches += 6;
             b.recs = s.g_recs; b.rec_counts = s.g_counts; b.blk_dp = s.g_dp; b.blk_pl = s.g_pl;
             CK(cudaMemcpyAsync(s.hg_counts, s.g_counts, 4 * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
@@ -1261,9 +1145,7 @@ extern "C" int vgl_submit(vgl_ctx* ctx, int slot, int64_t first_site_id, int32_t
     if (prm.host_output) CK(cudaMemcpyAsync(s.h_sites, s.d_sites, (size_t)n_sites * sizeof(vgl_site_out), cudaMemcpyDeviceToHost, st));
     if (tile_launch && !tile_status) s.h_totals[2] = 0; // the kernel posts the totals into the pinned words itself and raises no errors
     else CK(cudaMemcpyAsync(s.h_totals, s.d_totals, 8 * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-    if (narrow) CK(cudaMemcpyAsync(s.h_dpn, s.d_dpn, (size_t)cells * (ctx->narrow_bits / 8), cudaMemcpyDeviceToHost, st));
-    else if (bcf) {}
-    else if (prm.host_output) CK(cudaMemcpyAsync(s.h_dp, s.d_dp, (size_t)cells * 4, cudaMemcpyDeviceToHost, st));
+    CK(d2h_plane(ctx, s, P_DP, (size_t)cells));
     CK(cudaEventRecord(s.ev[EV_META], st));
     s.early_d2h = false;
     if (tile_launch && (prm.host_output == VGL_HOST_I32 || narrow)) {
@@ -1272,20 +1154,7 @@ extern "C" int vgl_submit(vgl_ctx* ctx, int slot, int64_t first_site_id, int32_t
         // instead of waiting for the host to come back for the totals
         const size_t g_up = (size_t)n_sites * (((size_t)S * 15 + 3) & ~(size_t)3), r_up = (size_t)n_sites * (((size_t)S * 5 + 3) & ~(size_t)3);
         CK(cudaEventRecord(s.ev[EV_D2H0], st));
-        if (s.d_gl) CK(cudaMemcpyAsync(s.h_gl, s.d_gl, g_up * 4, cudaMemcpyDeviceToHost, st));
-        if (s.d_gp) CK(cudaMemcpyAsync(s.h_gp, s.d_gp, g_up * 4, cudaMemcpyDeviceToHost, st));
-        if (narrow) {
-            const size_t w = (size_t)ctx->narrow_bits / 8;
-            if (s.d_pl8) CK(cudaMemcpyAsync(s.h_pl8, s.d_pl8, g_up, cudaMemcpyDeviceToHost, st));
-            if (s.d_adn) CK(cudaMemcpyAsync(s.h_adn, s.d_adn, r_up * w, cudaMemcpyDeviceToHost, st));
-            if (s.d_adfn) CK(cudaMemcpyAsync(s.h_adfn, s.d_adfn, r_up * w, cudaMemcpyDeviceToHost, st));
-            if (s.d_adrn) CK(cudaMemcpyAsync(s.h_adrn, s.d_adrn, r_up * w, cudaMemcpyDeviceToHost, st));
-        } else {
-            if (s.d_pl) CK(cudaMemcpyAsync(s.h_pl, s.d_pl, g_up * 4, cudaMemcpyDeviceToHost, st));
-            if (s.d_ad) CK(cudaMemcpyAsync(s.h_ad, s.d_ad, r_up * 4, cudaMemcpyDeviceToHost, st));
-            if (s.d_adf) CK(cudaMemcpyAsync(s.h_adf, s.d_adf, r_up * 4, cudaMemcpyDeviceToHost, st));
-            if (s.d_adr) CK(cudaMemcpyAsync(s.h_adr, s.d_adr, r_up * 4, cudaMemcpyDeviceToHost, st));
-        }
+        CK(d2h_planes(ctx, s, g_up, r_up));
         CK(cudaEventRecord(s.ev[EV_D2H1], st));
         s.early_d2h = true;
     }
@@ -1418,49 +1287,30 @@ extern "C" int vgl_wait(vgl_ctx* ctx, int slot, vgl_batch_out* out)
         if (s.had_d2h) CK(cudaEventElapsedTime(&d2h, s.ev[EV_D2H0], s.ev[EV_D2H1]));
         ms[VGL_T_D2H] = meta + d2h;
         CK(cudaEventElapsedTime(&ms[VGL_T_TOTAL], s.ev[EV_START], s.had_d2h ? s.ev[EV_D2H1] : s.ev[EV_META]));
-        if (getenv("VGL_TRACE") && (prm.host_output == VGL_HOST_BCF || prm.host_output == VGL_HOST_BGZF)) { // development: the kernel chain of the batch
-            float t_bcf = 0.f, t_z = 0.f, t_wait = 0.f;
-            cudaEventElapsedTime(&t_wait, s.ev[EV_H2D], s.ev[EV_SCAN]);
-            cudaEventElapsedTime(&t_bcf, s.ev[EV_EMIT], s.ev[EV_BCF]);
-            cudaEventElapsedTime(&t_z, s.ev[EV_BCF], s.ev[EV_KDONE]);
-            fprintf(stderr, "[vgl] batch: h2d %.2f, waited for the previous batch's kernels %.2f, simulate %.2f, serialise %.2f, compress %.2f ms\n",
-                    ms[VGL_T_H2D], t_wait, ms[VGL_T_EMIT], t_bcf, t_z);
-            static cudaEvent_t base = nullptr; // absolute timeline: the first traced batch's start
-            if (!base) base = s.ev[EV_START];
-            float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
-            cudaEventElapsedTime(&a0, base, s.ev[EV_START]);
-            cudaEventElapsedTime(&a1, base, s.ev[EV_SCAN]);
-            cudaEventElapsedTime(&a2, base, s.ev[EV_KDONE]);
-            cudaEventElapsedTime(&a3, base, s.ev[EV_D2H1]);
-            fprintf(stderr, "[vgl] timeline: submit %.2f  kernels %.2f .. %.2f  copies done %.2f\n", a0, a1, a2, a3);
-        }
     }
     s.waited = true;
     memset(out, 0, sizeof *out);
     out->n_sites = s.n_sites;
     out->n_samples = prm.n_samples;
+    // VGL_HOST_NONE: the device planes.  Else the host copies: none under VGL_HOST_BCF / BGZF (the host gets the serialised
+    // records), the narrowed ones where VGL_HOST_NARROW narrows a plane
     const bool h = prm.host_output != 0;
+    auto view = [&](int i) { return h ? s.plane[i].h : s.plane[i].d; };
     out->sites = h ? s.h_sites : s.d_sites;
-    out->dp = h ? s.h_dp : s.d_dp;
-    out->gl = h ? s.h_gl : s.d_gl;
-    out->pl = h ? s.h_pl : s.d_pl;
-    out->gp = h ? s.h_gp : s.d_gp;
-    out->ad = h ? s.h_ad : s.d_ad;
-    out->adf = h ? s.h_adf : s.d_adf;
-    out->adr = h ? s.h_adr : s.d_adr;
-    if (ctx->narrow_bits) { // the int32 planes stay on the device; the host gets the narrowed ones
-        out->dp = nullptr;
-        out->pl = out->ad = out->adf = out->adr = nullptr;
-        out->narrow_bits = ctx->narrow_bits;
-        out->pl_u8 = s.h_pl8;
-        out->dp_n = s.h_dpn;
-        out->ad_n = s.h_adn;
-        out->adf_n = s.h_adfn;
-        out->adr_n = s.h_adrn;
-    }
-    if (prm.host_output == VGL_HOST_BCF || prm.host_output == VGL_HOST_BGZF) { // the planes stay on the device; the host gets the serialised records
-        out->dp = nullptr; out->pl = out->ad = out->adf = out->adr = nullptr;
-        out->gl = out->gp = nullptr;
+    out->dp = (const int32_t*)view(P_DP);
+    out->gl = (const float*)view(P_GL);
+    out->pl = (const int32_t*)view(P_PL);
+    out->gp = (const float*)view(P_GP);
+    out->ad = (const int32_t*)view(P_AD);
+    out->adf = (const int32_t*)view(P_ADF);
+    out->adr = (const int32_t*)view(P_ADR);
+    out->narrow_bits = ctx->narrow_bits;
+    out->pl_u8 = (const uint8_t*)s.plane[P_PL].hn;
+    out->dp_n = s.plane[P_DP].hn;
+    out->ad_n = s.plane[P_AD].hn;
+    out->adf_n = s.plane[P_ADF].hn;
+    out->adr_n = s.plane[P_ADR].hn;
+    if (prm.host_output == VGL_HOST_BCF || prm.host_output == VGL_HOST_BGZF) {
         if (prm.host_output == VGL_HOST_BGZF) {
             out->bgzf = s.h_bgzf;
             out->bgzf_bytes = s.h_totals[4];
@@ -1484,7 +1334,7 @@ extern "C" int vgl_native_draws(vgl_ctx* ctx, int slot, int64_t first_site_id, i
     if (n_sites < 1 || n_sites > ctx->prm.max_batch_sites || first_site_id < 0) return fail(ctx, VGL_EINVAL, "n_sites / first_site_id out of range");
     Slot& s = ctx->slots[slot];
     if (s.submitted && !s.waited) return fail(ctx, VGL_ESTATE, "slot still in flight");
-    if (ctx->use_fused && !ctx->use_tile) return fail(ctx, VGL_ESTATE, "per-read draws do not exist under the count-level sampler (create the context with VGL_SAMPLER_PER_READ)");
+    if (ctx->plan.set == KS_FUSED_M1F) return fail(ctx, VGL_ESTATE, "per-read draws do not exist under the count-level sampler (create the context with VGL_SAMPLER_PER_READ)");
     const vgl_params& prm = ctx->prm;
     CK(cudaSetDevice(prm.device_id));
     cudaStream_t st = s.stream;
@@ -1492,14 +1342,14 @@ extern "C" int vgl_native_draws(vgl_ctx* ctx, int slot, int64_t first_site_id, i
     DevParams p;
     fill_params(ctx, s, first_site_id, n_sites, p);
     CK(cudaMemcpyAsync(s.d_gt, s.h_gt, (size_t)cells, cudaMemcpyHostToDevice, st));
-    const bool m2 = ctx->use_tile_m2 != 0; // the model-2 tile kernel's own sampler (read order matters there)
-    const bool m1t = ctx->use_tile != 0;    // the model-1 tile kernel's count-level sampler, listed read by read
-    if (m2) launch_tile_m2_draws(p, st, ctx->tile_m2_mode, 0, s.d_dp, nullptr, nullptr, nullptr);
-    else if (m1t) launch_tile_m1f_draws(p, st, 0, s.d_dp, nullptr, nullptr, nullptr, nullptr);
+    const bool m2 = ctx->plan.set == KS_TILE_M2;  // the model-2 tile kernel's own sampler (read order matters there)
+    const bool m1t = ctx->plan.set == KS_TILE_M1F; // the model-1 tile kernel's count-level sampler, listed read by read
+    if (m2) launch_tile_m2_draws(p, st, prm.error_qs, 0, s.dev(P_DP), nullptr, nullptr, nullptr);
+    else if (m1t) launch_tile_m1f_draws(p, st, 0, s.dev(P_DP), nullptr, nullptr, nullptr, nullptr);
     else launch_sim(p, st); // depths (and counts, unused here)
     ctx->launches += 1;
     s.dr_depths.resize((size_t)cells);
-    CK(cudaMemcpyAsync(s.dr_depths.data(), s.d_dp, (size_t)cells * 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(s.dr_depths.data(), s.dev(P_DP), (size_t)cells * 4, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     s.dr_off.resize((size_t)cells + 1);
     s.dr_off[0] = 0;
@@ -1515,11 +1365,11 @@ extern "C" int vgl_native_draws(vgl_ctx* ctx, int slot, int64_t first_site_id, i
     CK(cudaMemsetAsync(d_e, 0, nr * 8 + 16, st));
     CK(cudaMemcpyAsync(d_off, s.dr_off.data(), ((size_t)cells + 1) * 8, cudaMemcpyHostToDevice, st));
     if (m2) {
-        launch_tile_m2_draws(p, st, ctx->tile_m2_mode, 1, nullptr, d_off, d_u8, d_u8 + 2 * nr);
+        launch_tile_m2_draws(p, st, prm.error_qs, 1, nullptr, d_off, d_u8, d_u8 + 2 * nr);
         // the class table holds the score the GL uses: export it as both the raw and the adjusted score
         if (nr) CK(cudaMemcpyAsync(d_u8 + 3 * nr, d_u8 + 2 * nr, nr, cudaMemcpyDeviceToDevice, st));
     } else if (m1t) {
-        launch_tile_m1f_draws(p, st, 1, s.d_dp, d_off, d_u8, d_u8 + nr, d_u8 + 4 * nr);
+        launch_tile_m1f_draws(p, st, 1, s.dev(P_DP), d_off, d_u8, d_u8 + nr, d_u8 + 4 * nr);
     } else {
         launch_draws(p, st, d_off, d_u8, d_u8 + nr, d_u8 + 2 * nr, d_u8 + 3 * nr, d_u8 + 4 * nr, d_e);
     }

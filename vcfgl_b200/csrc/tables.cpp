@@ -640,4 +640,118 @@ bool bcf_fmt_blocks_tile(const uint8_t* p, uint64_t len, uint32_t n_fmt, int64_t
     return p == end;
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// The kernel set of a context
+const char* kernel_set_name(KernelSet k)
+{
+    static const char* const names[] = {"k_sim+k_site+k_scan+k_emit", "k_fused_m1f", "k_tile_m1f", "k_tile_m2", "k_truth_site+k_scan+k_truth_emit"};
+    return names[k];
+}
+
+namespace {
+// the model-2 tile kernel's tables: false when it cannot take the run (the per-read kernels keep the reference's behaviour)
+bool plan_tile_m2(const vgl_params& p, RunPlan* k, PlanTables* tab)
+{
+    std::vector<double> consts; // (homT, het, homF) per quality score in use
+    if (p.error_qs == 2) {
+        std::vector<int> qv;
+        tab->qcls = qs_class_table(k->beta_a, k->beta_b, (p.adjust_qs & 1) ? p.adjust_by : 0.0, p.n_qs_bins > 0, k->bin_lut, k->bin_max, nullptr,
+                                   &qv, &k->q_dom, &k->q_minor);
+        if (tab->qcls.empty()) return false; // classes outside the bins / too many
+        k->q_dom_idx = (int)((tab->qcls[256 + k->q_dom] >> 16) & 0xFFu);
+        for (int q : qv) consts.insert(consts.end(), {kLutLog10Gl[0][q], kLutLog10Gl[1][q], kLutLog10Gl[2][q]});
+    } else
+        consts = {k->pre.homT, k->pre.het, k->pre.homF};
+    // the table-driven update needs constants that are negative (finite and non-zero, or -inf): see m2_f2d() in tile_m2.cu.
+    // Not so e.g. under --precise-gl 1 with --error-rate 0 (homT = 0).
+    if (!std::all_of(consts.begin(), consts.end(), [](double c) { return c < 0.0; })) return false;
+    k->m2_nq = (int)consts.size() / 3;
+    tab->m2_tab = m2_const_table(consts);
+    if (!m2_pure_table(consts, &tab->m2_pure)) tab->m2_pure.clear();
+    return true;
+}
+} // namespace
+
+int plan_run(const vgl_params& p, const double* depth_means, bool allow_tile, RunPlan* k, PlanTables* tab, const char** why)
+{
+    auto fail = [why](int rc, const char* msg) { *why = msg; return rc; };
+    // ---- derived run constants (vcfgl.cpp:1661-1766, rng.h:368-371)
+    if (precalc(p.error_rate, p.error_qs, p.gl_model, p.precise_gl, p.adjust_qs, p.adjust_by, p.n_qs_bins, p.qs_bins, &k->pre) != 0)
+        return fail(VGL_ERANGE, "the fixed quality score falls outside every --qs-bins range");
+    if (p.error_qs != 2) k->gl_mode = p.gl_model == 1 ? GL_M1_FIXED : GL_M2_FIXED;
+    else k->gl_mode = p.gl_model == 1 ? GL_M1_PERREAD : (p.precise_gl ? GL_M2_PRECISE : GL_M2_LUT);
+    if (p.error_qs != 0) {
+        const double m = p.error_rate, one_over = 1.0 / m;
+        k->beta_a = (((1.0 - m) / p.beta_variance) - one_over) * pow(m, 2);
+        k->beta_b = k->beta_a * (one_over - 1);
+        if (!(k->beta_a > 0.0) || !(k->beta_b > 0.0)) return fail(VGL_EINVAL, "beta shape parameters must be positive (rng.h:373-388)");
+    }
+    const uint32_t t = p.tag_mask;
+    k->sample_strand = (t & (VGL_TAG_I16 | VGL_TAG_FMT_ADF | VGL_TAG_FMT_ADR | VGL_TAG_INFO_ADF | VGL_TAG_INFO_ADR)) != 0;
+    k->need_cellq = p.error_qs == 2 && (t & (VGL_TAG_QS | VGL_TAG_I16));
+    k->need_tail = (t & VGL_TAG_I16) != 0;
+    for (int i = 0; i < p.n_qs_bins; ++i) // first matching range wins (vcfgl.cpp:57-64)
+        for (int q = p.qs_bins[i][0]; q <= p.qs_bins[i][1]; ++q)
+            if (q > k->bin_max) { k->bin_lut[q] = p.qs_bins[i][2]; k->bin_max = q; }
+    if (p.gl_model == 1) {
+        ErrmodTables em;
+        em.build(1.0 - p.gl1_theta); // io.cpp:1276
+        tab->m1_het = em.het_term();
+        if (k->gl_mode == GL_M1_FIXED) {
+            tab->m1_bsum = em.fixed_q_bsum((p.adjust_qs & 1) ? k->pre.adj_qs : k->pre.qs); // gl_methods.cpp:318
+            k->fast_div = ErrmodTables::scores_safe_for_fast_div(tab->m1_bsum, tab->m1_het) ? 1 : 0;
+        } else {
+            tab->fk = std::move(em.fk);
+            tab->beta = std::move(em.beta);
+        }
+    }
+    // ---- the depth law: 256-column alias tables when no cell can get more than 255 reads
+    tab->alias.assign(256, 0ull);
+    k->alias_ok = p.depth_mode == VGL_DEPTH_FIXED && p.depth_mean < 256.0;
+    if (p.depth_mode == VGL_DEPTH_POISSON) {
+        tab->pois_cdf = poisson_cdf_u64(p.depth_mean, 1024);
+        std::vector<unsigned long long> al = poisson_alias_u64(tab->pois_cdf); // empty: depth can exceed 255
+        if (!al.empty()) { tab->alias = std::move(al); k->alias_ok = true; }
+    }
+    if (p.depth_mode == VGL_DEPTH_POISSON_PER_SAMPLE) { // --depths-file: one alias table per distinct mean, a row index per sample
+        std::vector<double> means;
+        std::vector<unsigned long long> all;
+        k->alias_ok = true;
+        for (int sidx = 0; sidx < p.n_samples && k->alias_ok; ++sidx) {
+            const double m = depth_means[sidx];
+            size_t row = 0;
+            while (row < means.size() && means[row] != m) ++row;
+            if (row == means.size()) {
+                const std::vector<unsigned long long> al = poisson_alias_u64(poisson_cdf_u64(m, 1024));
+                if (al.empty() || means.size() >= 65535) { k->alias_ok = false; break; }
+                means.push_back(m);
+                all.insert(all.end(), al.begin(), al.end());
+            }
+            tab->alias_row.push_back((uint16_t)row);
+        }
+        if (k->alias_ok) tab->alias = std::move(all);
+        else tab->alias_row.clear();
+    }
+    // ---- the kernel set
+    const bool plane_ok = (size_t)p.max_batch_sites * (((size_t)p.n_samples * 15 + 3) & ~(size_t)3) < (1ull << 31); // G-shaped plane
+    // the fused single-kernel path: native RNG, GL model 1 with a run-constant qs, count-level sampler
+    const bool fused = k->gl_mode == GL_M1_FIXED && p.sampler != VGL_SAMPLER_PER_READ && !(t & (VGL_TAG_QS | VGL_TAG_I16)) && plane_ok;
+    if (p.sampler == VGL_SAMPLER_COUNTS && !fused) return fail(VGL_EINVAL, "count-level sampler unavailable for this configuration (plane too large)");
+    const bool tile = allow_tile && plane_ok && k->alias_ok && p.n_samples <= TILE_M1F_MAX_SAMPLES;
+    // k_tile_m1f takes the fused path's runs without strand tags, and its AUX variant those with QS / I16 / INFO ADF, ADR / GP /
+    // FORMAT ADF, ADR
+    const bool tile_m1f = tile && k->gl_mode == GL_M1_FIXED && p.sampler != VGL_SAMPLER_PER_READ && p.error_qs == 0 && k->fast_div &&
+                          ((t & TILE_M1F_AUX_TAGS) || (fused && !k->sample_strand));
+    // k_tile_m2: native RNG, GL model 2 with run constants or the qs class table (not --precise-gl 1 with --error-qs 2), tags
+    // within GL / PL / AD / DP / INFO AD, DP
+    const uint32_t m2_tags = VGL_TAG_GL | VGL_TAG_PL | VGL_TAG_FMT_AD | VGL_TAG_FMT_DP | VGL_TAG_INFO_AD | VGL_TAG_INFO_DP;
+    const bool tile_m2 = tile && p.gl_model == 2 && p.sampler == VGL_SAMPLER_AUTO && !(p.error_qs == 2 && p.precise_gl) && !(t & ~m2_tags);
+    if (p.depth_mode == VGL_DEPTH_INF) k->set = KS_TRUTH;
+    else if (tile_m1f) k->set = KS_TILE_M1F;
+    else if (tile_m2 && plan_tile_m2(p, k, tab)) k->set = KS_TILE_M2;
+    else if (fused) k->set = KS_FUSED_M1F;
+    k->aux = k->set == KS_TILE_M1F && (t & TILE_M1F_AUX_TAGS);
+    return VGL_OK;
+}
+
 } // namespace vgl

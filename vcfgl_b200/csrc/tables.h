@@ -3,7 +3,17 @@
 #include <stdint.h>
 #include <vector>
 
+#include "../../include/vgl.h"
+
 namespace vgl {
+
+enum GlMode : int {
+    GL_M1_FIXED = 0,   // gl_methods.cpp:304-369  model 1, one qs for every read -> depends on base counts only
+    GL_M1_PERREAD = 1, // gl_methods.cpp:233-302  model 1, per-read qs
+    GL_M2_FIXED = 2,   // gl_methods.cpp:4-69     model 2, run-constant homT/het/homF
+    GL_M2_LUT = 3,     // gl_methods.cpp:71-150   model 2, qs -> LUT
+    GL_M2_PRECISE = 4  // gl_methods.cpp:152-231  model 2, log10 of the per-read error probability
+};
 
 // samtools/bcftools "revised MAQ" error-model coefficients
 // (reference: htslib/errmod.c:51-125, errmod_init(1 - theta) at io.cpp:1276)
@@ -104,5 +114,46 @@ void bgzf_build_code(const uint32_t* hist, bool fixed, BgzfCode* out);
 // descriptor with the vector size, n_samples vectors) tile the `len` bytes at p.  Every byte read lies inside them, and the
 // device's parser (bcf.cu in_fmt_block) then walks n_fmt blocks without leaving the range.
 bool bcf_fmt_blocks_tile(const uint8_t* p, uint64_t len, uint32_t n_fmt, int64_t n_samples);
+
+// ---- the kernel set of a context (vgl_create), chosen from its parameters alone
+enum { TILE_M1F_MAX_SAMPLES = 60000 }; // largest S the tile kernels take (the slot arithmetic needs (S4 + block) * S4 < 2^32)
+// tags the AUX variant adds to the tile kernel's GL / PL / AD / DP / INFO AD, DP
+enum : uint32_t { TILE_M1F_AUX_TAGS = VGL_TAG_QS | VGL_TAG_I16 | VGL_TAG_INFO_ADF | VGL_TAG_INFO_ADR | VGL_TAG_GP | VGL_TAG_FMT_ADF | VGL_TAG_FMT_ADR };
+enum KernelSet : int {
+    KS_PER_READ,  // k_sim, k_site, k_scan, k_emit: every configuration (and every replayed batch)
+    KS_FUSED_M1F, // k_fused_m1f: GL model 1 with a run-constant qs, count-level sampler
+    KS_TILE_M1F,  // k_tile_m1f (tile_m1f.cu): the fused path's headline special case, depths from the alias table, --error-qs 0
+    KS_TILE_M2,   // k_tile_m2 (tile_m2.cu): GL model 2 with run constants (--error-qs 0/1) or the qs class table (--error-qs 2)
+    KS_TRUTH      // --depth inf (truth.cu): k_truth_site, k_scan, k_truth_emit
+};
+const char* kernel_set_name(KernelSet k); // as vgl_native_kernels() reports it
+
+struct RunPlan { // the run constants of a context and its kernel set
+    KernelSet set = KS_PER_READ;
+    bool aux = false; // KS_TILE_M1F: the AUX variant (a tag of TILE_M1F_AUX_TAGS is on)
+    int gl_mode = GL_M1_FIXED;
+    PreCalc pre;
+    double beta_a = 0, beta_b = 0;
+    int sample_strand = 0, need_cellq = 0, need_tail = 0;
+    uint8_t bin_lut[256] = {};
+    int bin_max = -1;
+    int fast_div = 0;             // GL_M1_FIXED: the 3-instruction /10 is exact for every score
+    bool alias_ok = false;        // the depth law fits a 256-column alias table: no cell holds more than 255 reads
+    int q_dom = 0, q_dom_idx = 0; // KS_TILE_M2 with --error-qs 2: the dominant quality class (qs_class_table)
+    double q_minor = 0.0;
+    int m2_nq = 0;                // KS_TILE_M2: quality scores in m2_tab
+};
+struct PlanTables { // host tables the context uploads for its kernel set
+    std::vector<double> m1_het, m1_bsum, fk, beta; // GL model 1 (ErrmodTables)
+    std::vector<unsigned long long> pois_cdf;      // VGL_DEPTH_POISSON
+    std::vector<unsigned long long> alias;         // tile kernels: [rows][256] Walker alias tables of the depth law
+    std::vector<uint16_t> alias_row;               // --depths-file: each sample's row in alias
+    std::vector<uint32_t> qcls;                    // KS_TILE_M2, --error-qs 2: qs_class_table()
+    std::vector<double> m2_tab;                    // KS_TILE_M2: m2_const_table()
+    std::vector<float> m2_pure;                    // KS_TILE_M2: m2_pure_table(), when valid
+};
+// Fills the default-constructed *plan and *tab.  VGL_OK, or VGL_ERANGE / VGL_EINVAL with the reason in *why.  depth_means:
+// [n_samples] under VGL_DEPTH_POISSON_PER_SAMPLE.  allow_tile = false keeps the tile kernels out.
+int plan_run(const vgl_params& p, const double* depth_means, bool allow_tile, RunPlan* plan, PlanTables* tab, const char** why);
 
 } // namespace vgl

@@ -956,7 +956,7 @@ static void launch_tile_t(const DevParams& p, cudaStream_t st, int n_sms)
     else launch_tile_p<GEN, BIG, AUX, false, false>(p, st, n_sms);
 }
 
-// aux: QS / I16 / INFO ADF, ADR wanted (tile_m1f_aux_tags)
+// aux: QS / I16 / INFO ADF, ADR wanted (TILE_M1F_AUX_TAGS)
 void launch_tile_m1f(const DevParams& p, cudaStream_t st, int n_sms, bool aux)
 {
     const bool all3 = p.gl && p.pl && p.ad, big = tile_m1f_scratch_words(p.S, 1) > 0;
@@ -1030,11 +1030,6 @@ void launch_tile_m1f_draws(const DevParams& p, cudaStream_t st, int pass, int32_
     k_tile_m1f_draws<<<grid, 128, 0, st>>>(p, pass, depths, off, bases, strands, tails);
 }
 
-// tags the AUX variant adds to the tile kernel's GL / PL / AD / DP / INFO AD, DP
-uint32_t tile_m1f_aux_tags() { return VGL_TAG_QS | VGL_TAG_I16 | VGL_TAG_INFO_ADF | VGL_TAG_INFO_ADR | VGL_TAG_GP | VGL_TAG_FMT_ADF | VGL_TAG_FMT_ADR; }
-
-// largest S the tile kernel takes (the slot arithmetic needs (S4 + block) * S4 < 2^32)
-int tile_m1f_max_samples() { return 60000; }
 int tile_m1f_sites_per_tile(int S)
 {
     const int S4 = (S + 3) & ~3;

@@ -10,14 +10,6 @@
 
 namespace vgl {
 
-enum GlMode : int {
-    GL_M1_FIXED = 0,   // gl_methods.cpp:304-369  model 1, one qs for every read -> depends on base counts only
-    GL_M1_PERREAD = 1, // gl_methods.cpp:233-302  model 1, per-read qs
-    GL_M2_FIXED = 2,   // gl_methods.cpp:4-69     model 2, run-constant homT/het/homF
-    GL_M2_LUT = 3,     // gl_methods.cpp:71-150   model 2, qs -> LUT
-    GL_M2_PRECISE = 4  // gl_methods.cpp:152-231  model 2, log10 of the per-read error probability
-};
-
 // per-cell record written by the simulate kernel, read by the site and emit kernels (16 B)
 struct __align__(16) CellRec {
     uint16_t ad[4];  // reads per observed base A,C,G,T
@@ -194,7 +186,6 @@ void launch_tile_m1f(const DevParams& p, cudaStream_t st, int n_sms, bool aux);
 int build_m1f_pure_table(const double* d_bsum, const double* d_het, void* out, cudaStream_t st);
 void launch_tile_m1f_draws(const DevParams& p, cudaStream_t st, int pass, int32_t* depths, const int64_t* off, uint8_t* bases, uint8_t* strands,
                            uint8_t* tails);
-uint32_t tile_m1f_aux_tags();
 void launch_tile_m2(const DevParams& p, cudaStream_t st, int n_sms, int mode);
 size_t tile_m2_row_words(int S, int n_sms);
 size_t tile_m2_park_floats(int S, int n_sms);
@@ -202,7 +193,6 @@ void launch_tile_m2_draws(const DevParams& p, cudaStream_t st, int mode, int pas
                           uint8_t* qs);
 void launch_narrow(const int32_t* src, void* dst, int bits, bool is_pl, const int64_t* n_dev, int64_t n_fixed, int64_t cap, int32_t* status,
                    cudaStream_t st, int n_sms);
-int tile_m1f_max_samples();
 int tile_m1f_sites_per_tile(int S);
 size_t tile_m1f_scratch_words(int S, int n_sms);
 void launch_draws(const DevParams& p, cudaStream_t st, const int64_t* off, uint8_t* bases, uint8_t* strands, uint8_t* qs,
