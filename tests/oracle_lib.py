@@ -183,14 +183,53 @@ class Oracle:
                          d.em_sample, d.em_n, d.em_codes)
 
 
-def check_sites_on_draws(a, S, hap, native, rp, gl_rtol=0.0):
+F32_MISSING_BITS = 0x7F800001      # VGO_MISSING_F32_BITS (bcf_float_missing)
+
+
+def _bits(x):
+    return np.ascontiguousarray(x, dtype=np.float32).view(np.uint32)
+
+
+def check_gp(gp, gl_oracle, gp_oracle, fmt_dp, G):
+    """FORMAT/GP of one site ([S * G] float32) against
+    (a) a float64 reference made from the oracle's GL, independent of the float order of oracle and kernel:
+        ref = 10^gl / sum(10^gl) per sample, |gp - ref| <= (G + 2) 2^-24 ref + 2^-149 -- the float rounding of each term,
+        of the float sum of G positive terms and of the division; 2^-149 covers a subnormal GP (GL < -38);
+    (b) the oracle's GP: bit-equal or 1 float ulp apart (the device takes exp10 in double, the oracle libm pow: the two may
+        round to different floats);
+    (c) the missing value exactly in the samples with FORMAT/DP == 0.
+    Returns (values bit-equal to the oracle, values compared)."""
+    gp = _bits(gp).reshape(-1, G)
+    want = _bits(gp_oracle).reshape(-1, G)
+    assert gp.shape == want.shape, (gp.shape, want.shape)
+    dp0 = np.asarray(fmt_dp) == 0
+    miss = gp == F32_MISSING_BITS
+    assert (miss == dp0[:, None]).all(), ("GP missing where FORMAT/DP > 0, or set where FORMAT/DP == 0", np.nonzero(miss != dp0[:, None]))
+    have = ~dp0
+    got = gp[have].view(np.float32).astype(np.float64)
+    e = 10.0 ** np.asarray(gl_oracle, np.float32).reshape(-1, G)[have].astype(np.float64)
+    ref = e / e.sum(axis=1, keepdims=True)
+    bound = (G + 2) * 2.0 ** -24 * ref + 2.0 ** -149
+    bad = ~(np.abs(got - ref) <= bound)
+    assert not bad.any(), ("GP off the float64 reference", got[bad], ref[bad])
+    ulps = np.abs(gp[have].astype(np.int64) - want[have].astype(np.int64))     # both non-negative floats: bits are monotonic
+    assert (ulps <= 1).all(), ("GP more than 1 ulp from the oracle", got[ulps > 1], want[have][ulps > 1].view(np.float32))
+    return int((ulps == 0).sum()), int(ulps.size)
+
+
+def check_sites_on_draws(a, S, hap, native, rp, gl_rtol=0.0, idx=None, orc=None, gp_share=None):
     """The oracle run on a batch's own draws (vgl_native_draws: `rp`) must give the tags the kernels emitted for that batch:
-    native[i] = Batch.site(i) of site i, hap = int8 [n_sites, 2S] true genotypes.  GL bit for bit, or (gl_rtol > 0) within
-    that relative tolerance where the bits differ.  Returns the number of written sites compared."""
-    orc = Oracle(a, S)
+    native[i] = Batch.site(i) of site i, hap = int8 [n_sites, 2S] true genotypes.  Every field of the record (n_alleles*,
+    INFO/DP, INFO AD family, QS, I16; the allele maps where INFO/DP > 0) and every plane asked for (FORMAT/DP, GL, PL, the
+    FORMAT AD family; GP through check_gp).  A plane the arguments ask for that the batch does not return is a failure.  GL bit
+    for bit, or (gl_rtol > 0) within that relative tolerance where the bits differ.  `idx`: the sites to compare (default:
+    all); `orc`: an Oracle of (a, S) to reuse; `gp_share`: a [bit-equal, compared] pair the GP counts are added to.
+    Returns the number of written sites compared."""
+    orc = orc or Oracle(a, S)
     off = rp["read_offsets"]
     n_cmp = 0
-    for i, d in enumerate(native):
+    for i in (range(len(native)) if idx is None else idx):
+        d = native[i]
         sl = slice(off[i * S], off[(i + 1) * S])
         o = orc.site(hap[i], rp["depths"][i * S:(i + 1) * S], rp["bases"][sl], rp["strands"][sl],
                      None if rp["qs"] is None else rp["qs"][sl].astype(np.int32),
@@ -198,21 +237,38 @@ def check_sites_on_draws(a, S, hap, native, rp, gl_rtol=0.0):
                      None if rp["error_probs"] is None else rp["error_probs"][sl],
                      rp["tail_dists"][sl].astype(np.int32) if a.add_i16 else None)
         assert o["ret"] == d["skip_code"], i
+        if a.add_fmt_dp:
+            assert d.get("fmt_dp") is not None, (i, "fmt_dp")
+            assert np.array_equal(o["fmt_dp"], d["fmt_dp"]), (i, "fmt_dp")
         if o["ret"] != 0:
             continue
         assert o["n_alleles"] == d["n_alleles"] and o["n_genotypes"] == d["n_genotypes"], i
+        assert o["n_alleles_observed"] == d["n_alleles_observed"], (i, o["n_alleles_observed"], d["n_alleles_observed"])
+        assert o["info_dp"] == d["info_dp"], (i, o["info_dp"], d["info_dp"])
+        if o["info_dp"] > 0:
+            assert np.array_equal(o["alleles2acgt"], d["alleles2acgt"]), (i, o["alleles2acgt"], d["alleles2acgt"])
+            assert np.array_equal(o["acgt2alleles"], d["acgt2alleles"]), (i, o["acgt2alleles"], d["acgt2alleles"])
         for key in ("pl", "fmt_ad", "fmt_adf", "fmt_adr", "info_ad", "info_adf", "info_adr"):
-            if not getattr(a, "add_" + key) or d.get(key) is None:
+            if not getattr(a, "add_" + key):
                 continue
+            assert d.get(key) is not None, (i, key, "asked for, not returned")
             assert np.array_equal(o[key], d[key]), (i, key, o[key], d[key])
-        same = o["gl"].view(np.uint32) == np.ascontiguousarray(d["gl"]).view(np.uint32)   # missing (a NaN payload) compares by bits
-        if gl_rtol > 0:
-            with np.errstate(invalid="ignore"):
-                same |= np.abs(o["gl"].astype(np.float64) - d["gl"]) <= gl_rtol * np.abs(d["gl"].astype(np.float64))
-        assert same.all(), i
+        if a.add_gl:
+            assert d.get("gl") is not None, (i, "gl", "asked for, not returned")
+            same = o["gl"].view(np.uint32) == _bits(d["gl"])   # missing (a NaN payload) compares by bits
+            if gl_rtol > 0:
+                with np.errstate(invalid="ignore"):
+                    same |= np.abs(o["gl"].astype(np.float64) - d["gl"]) <= gl_rtol * np.abs(d["gl"].astype(np.float64))
+            assert same.all(), i
+        if a.add_gp:
+            assert d.get("gp") is not None, (i, "gp", "asked for, not returned")
+            eq, n = check_gp(d["gp"], o["gl"], o["gp"], o["fmt_dp"], o["n_genotypes"])
+            if gp_share is not None:
+                gp_share[0] += eq
+                gp_share[1] += n
         if a.add_qs:
-            assert np.array_equal(o["qs"].view(np.uint32), np.ascontiguousarray(d["qs"]).view(np.uint32)), i
+            assert np.array_equal(o["qs"].view(np.uint32), _bits(d["qs"])), i
         if a.add_i16:
-            assert np.array_equal(o["i16"].view(np.uint32), np.ascontiguousarray(d["i16"]).view(np.uint32)), (i, o["i16"], d["i16"])
+            assert np.array_equal(o["i16"].view(np.uint32), _bits(d["i16"])), (i, o["i16"], d["i16"])
         n_cmp += 1
     return n_cmp

@@ -51,7 +51,8 @@ def test_native_tags_match_oracle_on_own_draws(name):
     self_replay(name, SELF_CASES[name], 1, S, n_sites)
 
 
-def self_replay(name, argv, sampler, S, n_sites, kernels=None, qs_bins=None, depths=None):
+def self_replay(name, argv, sampler, S, n_sites, kernels=None, qs_bins=None, depths=None, gp_share=None):
+    """`gp_share`: a [bit-equal, compared] pair the GP values compared with the oracle are added to"""
     a = vargs.parse_args(argv.split(), qs_bins=qs_bins, depths=depths)
     hap = synth.sfs_genotypes(n_sites, S, 99, missing_rate=0.05) if S > 1 else \
         np.random.default_rng(1).integers(0, 2, (n_sites, 2)).astype(np.int8)
@@ -69,7 +70,13 @@ def self_replay(name, argv, sampler, S, n_sites, kernels=None, qs_bins=None, dep
     assert np.array_equal(rp["depths"], b.dp)
     # (a) oracle on the kernel's draws (the oracle needs the kept-read capture for depth > 255; covered by (b) + golden d300 cases)
     if "deep" not in name:
-        assert oracle_lib.check_sites_on_draws(a, S, hap, native, rp, gl_rtol=1e-6 if name == "gl2_precise" else 0.0) > 0
+        share = [0, 0]
+        assert oracle_lib.check_sites_on_draws(a, S, hap, native, rp, gl_rtol=1e-6 if name == "gl2_precise" else 0.0, gp_share=share) > 0
+        if gp_share is not None:
+            gp_share[0] += share[0]
+            gp_share[1] += share[1]
+        if a.add_gp:
+            print("%s: GP bit-equal to the oracle: %d of %d (%s)" % (name, share[0], share[1], ctx.native_kernels()))
     # (b) replay of the kernel's draws through the C ABI, in two batches with different slots sizes
     if "deep" not in name:
         ctx.submit(0, 7, n_sites, replay=rp)
@@ -77,7 +84,7 @@ def self_replay(name, argv, sampler, S, n_sites, kernels=None, qs_bins=None, dep
         for i in range(n_sites):
             d, e = native[i], b2.site(i)
             assert d["skip_code"] == e["skip_code"]
-            if d["skip_code"] == 0:
+            if d["skip_code"] == 0 and a.add_gl:
                 assert np.array_equal(u32(d["gl"]), u32(e["gl"])), (name, i)
     # (c) batch-size independence: the same sites in two half batches give identical tags
     h = n_sites // 2
@@ -88,7 +95,9 @@ def self_replay(name, argv, sampler, S, n_sites, kernels=None, qs_bins=None, dep
         d, e = native[i], b3.site(i - h)
         assert d["skip_code"] == e["skip_code"]
         if d["skip_code"] == 0:
-            assert np.array_equal(u32(d["gl"]), u32(e["gl"])), (name, i)
+            for key in ("gl", "gp"):
+                if getattr(a, "add_" + key):
+                    assert np.array_equal(u32(d[key]), u32(e[key])), (name, i, key)
             assert np.array_equal(d["fmt_dp"], e["fmt_dp"])
     ctx.close()
 

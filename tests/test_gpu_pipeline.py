@@ -26,6 +26,7 @@ import torch
 import oracle_lib
 from bcf_util import bo
 import truth_util as tu
+from device_util import device_plane
 from test_gpu_bgzf import inflate_all, split_blocks
 from vcfgl_b200 import args as vargs
 from vcfgl_b200 import capi, synth
@@ -68,19 +69,6 @@ def batch_list(S, B, seed, truth=False, reps=4):
             out.append((first, synth.pack_gt(hap), hap))
             first += n + (0 if j % 3 else 1000003 * (r + 1))      # gaps between the site ids of some batches
     return out
-
-
-def device_plane(ptr, typestr, n):
-    """a copy of n elements of a device plane, taken through its CUDA array interface"""
-    if not ptr:
-        return None
-    dt = np.dtype(typestr)
-    if n == 0:
-        return np.zeros(0, dt)
-
-    class Plane:
-        __cuda_array_interface__ = {"shape": (int(n),), "typestr": typestr, "data": (ptr, False), "version": 3}
-    return torch.as_tensor(Plane(), device="cuda").clone().cpu().numpy()
 
 
 def collect(ctx, slot, mode, disc):
@@ -141,7 +129,9 @@ def site_dicts(r, S):
     out = []
     for i, s in enumerate(r["sites"]):
         A, G = int(s["n_alleles"]), int(s["n_genotypes"])
-        d = dict(skip_code=int(s["skip_code"]), n_alleles=A, n_genotypes=G, alleles2acgt=s["alleles2acgt"][:5].astype(np.int32),
+        d = dict(skip_code=int(s["skip_code"]), n_alleles=A, n_alleles_observed=int(s["n_alleles_observed"]), n_genotypes=G,
+                 alleles2acgt=s["alleles2acgt"][:5].astype(np.int32), acgt2alleles=s["acgt2alleles"][:5].astype(np.int32),
+                 info_dp=int(s["info_dp"]),
                  info_ad=s["info_ad"][:A], info_adf=s["info_adf"][:A], info_adr=s["info_adr"][:A], qs=s["qs"][:A], i16=s["i16"],
                  fmt_dp=None if r["dp"] is None else r["dp"][i * S:(i + 1) * S])
         if d["skip_code"] == 0:

@@ -4,8 +4,10 @@ import ctypes as C
 
 import pytest
 
+import bench
 import test_gpu_narrow
 import test_gpu_native
+import test_gpu_oracle_shapes as shapes
 import test_gpu_pipeline
 import test_gpu_tile_aux
 import test_gpu_tile_m2
@@ -107,6 +109,26 @@ def test_pipeline_cases(plan, name):
 def test_narrow_cases(plan, name):
     argv, S, n_sites, kernels, _ = test_gpu_narrow.NATIVE[name]
     assert plan(argv, S, n_sites) == kernels
+
+
+@pytest.mark.parametrize("name", sorted(shapes.XTRA_CASES))
+def test_oracle_shapes_xtra_cases(plan, name):
+    _, S, _, _ = shapes.XTRA_CASES[name]
+    assert plan(shapes.xtra_argv(name), S, shapes.XTRA_S[S]) == TILE
+
+
+@pytest.mark.parametrize("fam", shapes.FAM)
+@pytest.mark.parametrize("S,B", [(4, 65), (37, 3 * 148 * 8 * 32), (2049, 3 * 148 * 8), (60000, 3)])
+def test_oracle_shapes_families(plan, fam, S, B):
+    """the families of the geometry sweep and of the many-tiles batches (148 SMs)"""
+    argv, kernels, bins = shapes.FAMILIES[fam]
+    assert plan("--seed 1 -d 2 " + argv, S, B, qs_bins=bins) == kernels
+
+
+@pytest.mark.parametrize("name", sorted(shapes.BENCH_KERNELS))
+def test_oracle_shapes_benched(plan, name):
+    wl = bench.Workload(name)
+    assert plan(["--seed", "42"] + wl.argv, wl.S, wl.B, qs_bins=wl.bins) == shapes.BENCH_KERNELS[name]
 
 
 # ---- the edges of the rules
