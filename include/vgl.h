@@ -297,7 +297,7 @@ typedef struct vgl_draws {
     const int32_t* depths;       /* [n_cells] (0 where the genotype is missing) */
     const int64_t* read_offsets; /* [n_cells + 1] */
     const uint8_t *bases, *strands, *qs, *adj_qs, *tail_dists; /* [n_reads]; qs/adj_qs only with --error-qs 2 */
-    const double* error_probs;   /* [n_reads], --error-qs 2 */
+    const double* error_probs;   /* [n_reads]: --error-qs 2 the read's own, --error-qs 1 its site's error rate */
 } vgl_draws;
 int vgl_native_draws(vgl_ctx* ctx, int slot, int64_t first_site_id, int32_t n_sites, vgl_draws* out);
 

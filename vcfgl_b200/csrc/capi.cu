@@ -1344,7 +1344,7 @@ extern "C" int vgl_native_draws(vgl_ctx* ctx, int slot, int64_t first_site_id, i
     CK(cudaMemcpyAsync(s.d_gt, s.h_gt, (size_t)cells, cudaMemcpyHostToDevice, st));
     const bool m2 = ctx->plan.set == KS_TILE_M2;  // the model-2 tile kernel's own sampler (read order matters there)
     const bool m1t = ctx->plan.set == KS_TILE_M1F; // the model-1 tile kernel's count-level sampler, listed read by read
-    if (m2) launch_tile_m2_draws(p, st, prm.error_qs, 0, s.dev(P_DP), nullptr, nullptr, nullptr);
+    if (m2) launch_tile_m2_draws(p, st, prm.error_qs, 0, s.dev(P_DP), nullptr, nullptr, nullptr, nullptr);
     else if (m1t) launch_tile_m1f_draws(p, st, 0, s.dev(P_DP), nullptr, nullptr, nullptr, nullptr);
     else launch_sim(p, st); // depths (and counts, unused here)
     ctx->launches += 1;
@@ -1365,7 +1365,7 @@ extern "C" int vgl_native_draws(vgl_ctx* ctx, int slot, int64_t first_site_id, i
     CK(cudaMemsetAsync(d_e, 0, nr * 8 + 16, st));
     CK(cudaMemcpyAsync(d_off, s.dr_off.data(), ((size_t)cells + 1) * 8, cudaMemcpyHostToDevice, st));
     if (m2) {
-        launch_tile_m2_draws(p, st, prm.error_qs, 1, nullptr, d_off, d_u8, d_u8 + 2 * nr);
+        launch_tile_m2_draws(p, st, prm.error_qs, 1, nullptr, d_off, d_u8, d_u8 + 2 * nr, d_e);
         // the class table holds the score the GL uses: export it as both the raw and the adjusted score
         if (nr) CK(cudaMemcpyAsync(d_u8 + 3 * nr, d_u8 + 2 * nr, nr, cudaMemcpyDeviceToDevice, st));
     } else if (m1t) {
@@ -1396,7 +1396,7 @@ extern "C" int vgl_native_draws(vgl_ctx* ctx, int slot, int64_t first_site_id, i
     out->qs = prm.error_qs == 2 ? s.dr_qs.data() : nullptr;
     out->adj_qs = prm.error_qs == 2 && prm.adjust_qs ? s.dr_adjqs.data() : nullptr;
     out->tail_dists = s.dr_tails.data();
-    out->error_probs = prm.error_qs == 2 ? s.dr_eprob.data() : nullptr;
+    out->error_probs = prm.error_qs != 0 ? s.dr_eprob.data() : nullptr; // --error-qs 1: each read carries its site's rate
     return VGL_OK;
 }
 

@@ -112,7 +112,7 @@ __device__ __forceinline__ CellCounts sample_counts(const CountsParams& cp, int6
     int E = 0;
     if (e > 0.0) {
         const float p0 = exp2f((float)n * l2);
-        const float uf = ((float)(w.z >> 8) + 0.5f) * 5.9604645e-08f; // 24-bit uniform in (0,1)
+        const float uf = ((float)(w.z >> 8) + 0.5f) * 5.9604645e-08f; // 24-bit uniform in (0,1]: the top word rounds to 1.0f
         if (uf > 0.998f) {
             // the upper tail: a float CDF saturates at 1.0f and a 24-bit uniform cannot fall into events rarer than 6e-8 per cell
             // (five errors in ten reads at e = 0.01) -- exact inversion in double with 64 random bits

@@ -97,6 +97,8 @@ __global__ void __launch_bounds__(VGL_BLOCK) k_draws(const __grid_constant__ Dev
             qs[o + i] = (uint8_t)(r.qs < 0 ? 0 : r.qs);
             adjqs[o + i] = (uint8_t)(r.adjqs < 0 ? 0 : r.adjqs);
             eprob[o + i] = r.eprob;
+        } else if (p.error_qs == 1) {
+            eprob[o + i] = cs.e_pick; // the site's error rate
         }
     }
 }

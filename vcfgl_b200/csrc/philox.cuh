@@ -6,6 +6,7 @@
 // (north_star; replaces the reference's four sequential libc streams,
 // SURVEY.md 3.4: rng.h:8-12, io.cpp:1047-1061).
 #pragma once
+#include <math.h>
 #include <stdint.h>
 
 namespace vgl {
@@ -71,11 +72,12 @@ __host__ __device__ __forceinline__ u32x4 draw(Key key, int64_t site, uint32_t s
 
 // uniform in (0,1), 32-bit resolution, never 0 or 1
 __host__ __device__ __forceinline__ double u01_32(uint32_t w) { return ((double)w + 0.5) * 2.3283064365386963e-10; }
-// uniform in (0,1), 53-bit resolution
+// uniform in (0,1), 53-bit resolution, never 0 or 1: 2^53 - 1 + 0.5 rounds to 2^53, so the top value is clamped to the
+// largest double below 1 (no other value reaches it)
 __host__ __device__ __forceinline__ double u01_53(uint32_t hi, uint32_t lo)
 {
     const uint64_t v = ((uint64_t)hi << 21) ^ (uint64_t)(lo >> 11); // 53 bits
-    return ((double)v + 0.5) * 1.1102230246251565e-16;
+    return fmin(((double)v + 0.5) * 1.1102230246251565e-16, 0x1.fffffffffffffp-1);
 }
 
 // sequential stream of 32-bit words for rejection samplers (one Philox block per 4 words)

@@ -144,12 +144,14 @@ std::vector<uint32_t> binomial_cdf4_u32(double e)
 {
     std::vector<uint32_t> t(256 * 4, 0xFFFFFFFFu);
     if (!(e > 0.0)) return t; // never an error: every u < 2^32-1 gives E = 0
-    const long double le = logl((long double)e), l1 = log1pl(-(long double)e);
+    // P(E = j) by the ratio recurrence from (1 - e)^n: every step is one rounded operation, so a CDF that is a short dyadic
+    // fraction (e = 1/4, 1/2) comes out exact and its floor is not one short
+    const long double E = e, Q = 1.0L - E;
     for (int n = 0; n < 256; ++n) {
-        long double cdf = 0.0L;
+        long double cdf = 0.0L, pj = powl(Q, n);
         for (int j = 0; j < 4 && j <= n; ++j) {
-            const long double lp = lgammal(n + 1.0L) - lgammal(j + 1.0L) - lgammal(n - j + 1.0L) + j * le + (n - j) * l1;
-            cdf += expl(lp);
+            if (j > 0) pj = pj * (n - j + 1) * E / (j * Q);
+            cdf += pj;
             const long double sc = cdf * 4294967296.0L;
             t[n * 4 + j] = sc >= 4294967295.0L ? 0xFFFFFFFFu : (uint32_t)sc;
         }

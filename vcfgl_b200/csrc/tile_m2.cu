@@ -140,7 +140,7 @@ __device__ __forceinline__ uint32_t m2_cell_fixed(const DevParams& p, const M2Rn
     if (SITE_E) {
         if (se.e > 0.0) {
             const float p0 = exp2f((float)n * se.l2);
-            const float uf = ((float)(b0.z >> 8) + 0.5f) * 5.9604645e-08f;
+            const float uf = ((float)(b0.z >> 8) + 0.5f) * 5.9604645e-08f; // 24-bit uniform in (0,1]: the top word rounds to 1.0f
             if (se.l2 != 0.0f && p0 > 1e-30f) {
                 float pr = p0, cdf = p0;
                 while (uf > cdf && E < n) {
@@ -148,6 +148,11 @@ __device__ __forceinline__ uint32_t m2_cell_fixed(const DevParams& p, const M2Rn
                     cdf += pr;
                     ++E;
                 }
+                // The float CDF can end below uf: it often ends at 0.99999994f or lower, and the top word's uf is 1.0f.  The walk
+                // has then run to E = n; such a cell takes the exact inversion in double from the same word.  Sending every
+                // uf > 0.998f there, as sample_counts does, made k_tile_m2 12% slower on cfg3(i) (0.62 -> 0.70 ms per batch, B200
+                // at 1000 W): one lane in 500 takes it, so one warp-wide pass in 16 waits for a double-precision inversion.
+                if (uf > cdf) E = m2_binom_inversion(n, se.e, b0.z);
             } else {
                 E = m2_binom_inversion(n, se.e, b0.z);
             }
@@ -933,7 +938,8 @@ size_t tile_m2_park_floats(int S, int n_sms)
 }
 
 // ---- the sampler's per-read draws in the replay layout (vgl_native_draws): pass 0 writes the depths, pass 1 the reads
-__global__ void k_tile_m2_draws(const DevParams p, int mode, int pass, int32_t* depths, const int64_t* off, uint8_t* bases, uint8_t* qs)
+__global__ void k_tile_m2_draws(const DevParams p, int mode, int pass, int32_t* depths, const int64_t* off, uint8_t* bases, uint8_t* qs,
+                                double* eprob)
 {
     __shared__ __align__(16) unsigned char sm[2048 + 4096 + 2048];
     for (int i = threadIdx.x; i < 256; i += blockDim.x) {
@@ -977,6 +983,7 @@ __global__ void k_tile_m2_draws(const DevParams p, int mode, int pass, int32_t* 
         if (n > 64) b = m2_deep_base(p, site, sample, i, g0, g1, se.e);
         else b = (int)((w[i >> 4] >> (2 * (i & 15))) & 3u);
         bases[off[c] + i] = (uint8_t)b;
+        if (mode == 1) eprob[off[c] + i] = se.e; // the site's error rate
     }
     if (mode == 2) {
         if (n > 64) {
@@ -997,10 +1004,11 @@ __global__ void k_tile_m2_draws(const DevParams p, int mode, int pass, int32_t* 
     }
 }
 
-void launch_tile_m2_draws(const DevParams& p, cudaStream_t st, int mode, int pass, int32_t* depths, const int64_t* off, uint8_t* bases, uint8_t* qs)
+void launch_tile_m2_draws(const DevParams& p, cudaStream_t st, int mode, int pass, int32_t* depths, const int64_t* off, uint8_t* bases, uint8_t* qs,
+                          double* eprob)
 {
     const unsigned grid = (unsigned)((p.n_cells + 127) / 128);
-    k_tile_m2_draws<<<grid, 128, 0, st>>>(p, mode, pass, depths, off, bases, qs);
+    k_tile_m2_draws<<<grid, 128, 0, st>>>(p, mode, pass, depths, off, bases, qs, eprob);
 }
 
 } // namespace vgl

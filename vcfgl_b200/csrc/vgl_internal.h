@@ -190,7 +190,7 @@ void launch_tile_m2(const DevParams& p, cudaStream_t st, int n_sms, int mode);
 size_t tile_m2_row_words(int S, int n_sms);
 size_t tile_m2_park_floats(int S, int n_sms);
 void launch_tile_m2_draws(const DevParams& p, cudaStream_t st, int mode, int pass, int32_t* depths, const int64_t* off, uint8_t* bases,
-                          uint8_t* qs);
+                          uint8_t* qs, double* eprob);
 void launch_narrow(const int32_t* src, void* dst, int bits, bool is_pl, const int64_t* n_dev, int64_t n_fixed, int64_t cap, int32_t* status,
                    cudaStream_t st, int n_sms);
 int tile_m1f_sites_per_tile(int S);
